@@ -1,7 +1,7 @@
 /*
  * libsegger_b200 -- C ABI of the B200-native segger hot path.
  *
- * Every entry point is `extern "C"`, takes plain device pointers and sizes (no torch types),
+ * Every entry point (73) is `extern "C"`, takes plain device pointers and sizes (no torch types),
  * enqueues its work on the `stream` passed in (a cudaStream_t) and returns 0 on success or a
  * negative SGB_ERR_* code; the message is available from sgb_last_error() (thread-local).
  * The library never allocates, frees or retains device memory: outputs and workspaces are
@@ -399,6 +399,28 @@ SGB_API int sgb_tilecut_edges(const int32_t* eperm, const void* edge_index, int 
                       const void* src_pos, int pos_f64, const double* boxes, int T, const int64_t* src_keys,
                       const int64_t* src_ptr, const int64_t* dst_keys, const int64_t* dst_ptr, int64_t* ekeys, int32_t* pu,
                       int32_t* pv, uint8_t* mask, int32_t* slot_counts, void* stream);
+/* Quadtree tiling: QuadTreeTiling (data/tiling.py:198-235, cuSpatial leaves of <= max_tile_size points over all node
+ * positions) and TileFitDataset's tile label / training mask (data/tile_dataset.py:13-153).  Rules (oracle/quadtree_ref.py):
+ * root = (xmin, ymin, scale = max(x range, y range, or 1 if 0) / 2^D), D = max_depth in 1..15; every cell edge is
+ * xmin + c * scale in fp64; a point's cell is floor((x - xmin) / scale) corrected by +-1 so that the point lies in
+ * [edge(c), edge(c+1)), clamped to [0, 2^D - 1]; a quadrant at level L < D holding > max_tile_size points is split;
+ * tiles = non-empty unsplit quadrants in Morton order (x in the even key bits).
+ * sgb_quadtree_build: labels[n] = tile of each point; root[3] = (xmin, ymin, scale); per tile leaf_meta[3] = (Morton
+ *   prefix of 2*level bits, level, point count) and leaf_box[4] = (x0, y0, x1, y1); *n_leaves = tile count (leaf_cap >=
+ *   sgb_quadtree_max_leaves(n, max_tile_size, max_depth) rows are caller-allocated).
+ * sgb_quadtree_label: labels[n] = tile whose quadrant contains the point's cell (points outside the root clamp to the rim
+ *   cells), -1 when that cell lies in an empty quadrant.
+ * sgb_quadtree_fit_mask: mask[n] = point inside its own tile's box shrunk by margins[label] on every side (closed); 0 for
+ *   labels outside [0, n_leaves). */
+SGB_API int64_t sgb_quadtree_max_leaves(int64_t n, int64_t max_tile_size, int max_depth);
+SGB_API size_t sgb_quadtree_workspace_bytes(int64_t n, int64_t max_tile_size, int max_depth);
+SGB_API int sgb_quadtree_build(const void* pos, int pos_f64, int64_t n, int64_t max_tile_size, int max_depth, int32_t* labels,
+                       double* root, int32_t* leaf_meta, double* leaf_box, int64_t leaf_cap, int32_t* n_leaves, void* ws,
+                       size_t ws_bytes, void* stream);
+SGB_API int sgb_quadtree_label(const void* pts, int pos_f64, int64_t n, const double* root, int max_depth, const int32_t* leaf_meta,
+                       int n_leaves, int32_t* labels, void* stream);
+SGB_API int sgb_quadtree_fit_mask(const void* pos, int pos_f64, int64_t n, const int32_t* labels, const double* leaf_box,
+                          const double* margins, int n_leaves, uint8_t* mask, void* stream);
 /* batch[r] = k for out_off[k] <= r < out_off[k+1] (the PyG Batch.batch vector). */
 SGB_API int sgb_batch_vector(const int64_t* out_off, int K, int64_t total_rows, int64_t* batch, void* stream);
 /* `src_idx[mask], seg_idx[mask], max_sim[mask], gen_idx[mask]` of LitISTEncoder.predict_step

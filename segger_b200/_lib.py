@@ -113,6 +113,11 @@ _PROTOS = {
                                     c_i64, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "sgb_ranges_gather": (c_int, [c_vp, c_i64, c_vp, c_vp, c_int, c_i64, c_vp, c_vp]),
     "sgb_edges_collate": (c_int, [c_vp, c_int, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_i64, c_vp, c_i64, c_vp]),
+    "sgb_quadtree_max_leaves": (c_i64, [c_i64, c_i64, c_int]),
+    "sgb_quadtree_workspace_bytes": (c_sz, [c_i64, c_i64, c_int]),
+    "sgb_quadtree_build": (c_int, [c_vp, c_int, c_i64, c_i64, c_int, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_sz, c_vp]),
+    "sgb_quadtree_label": (c_int, [c_vp, c_int, c_i64, c_vp, c_int, c_vp, c_int, c_vp, c_vp]),
+    "sgb_quadtree_fit_mask": (c_int, [c_vp, c_int, c_i64, c_vp, c_vp, c_vp, c_int, c_vp, c_vp]),
     "sgb_batch_vector": (c_int, [c_vp, c_int, c_i64, c_vp, c_vp]),
     "sgb_dedupe_workspace_bytes": (c_sz, [c_i64]),
     "sgb_dedupe_max": (c_int, [c_vp, c_vp, c_vp, c_i64, c_int, c_vp, c_vp, c_vp, c_sz, c_vp]),

@@ -133,6 +133,111 @@ def _dev_i64(values: Sequence[int], device) -> Tensor:
 
 
 # ---------------------------------------------------------------------------------------------------------------------
+# quadtree tiles (QuadTreeTiling + TileFitDataset labels / masks)
+# ---------------------------------------------------------------------------------------------------------------------
+def _pos_arg(pos: Tensor) -> Tensor:
+    require_cuda(pos)
+    if pos.dim() != 2 or pos.size(1) != 2:
+        raise ValueError(f"positions must be [N, 2], got {tuple(pos.shape)}")
+    return (pos if pos.dtype in (torch.float32, torch.float64) else pos.float()).contiguous()
+
+
+def fit_margins(boxes: Tensor, margin: float) -> Tensor:
+    """Per-tile training margin (data/tiling.py:103-127): ``margin / 2**j`` with the smallest ``j >= 0`` that leaves the
+    box shrunk by it non-empty in both axes.  fp64 on the host, once per tiling; returned on the boxes' device."""
+    b = boxes.detach().to("cpu", torch.float64)
+    m = torch.full((b.size(0),), float(margin), dtype=torch.float64)
+    while True:
+        bad = (m > 0) & ~((b[:, 0] + m <= b[:, 2] - m) & (b[:, 1] + m <= b[:, 3] - m))
+        if not bool(bad.any()):
+            return m.to(boxes.device)
+        m = torch.where(bad, m / 2, m)
+
+
+class QuadTreeTiling:
+    """``QuadTreeTiling`` (data/tiling.py:198-235) without cuSpatial: quadtree leaves holding <= ``max_tile_size`` points
+    over ``positions`` -- an [N, 2] fp32 / fp64 CUDA tensor, or a dict of them per node type (all node positions, as
+    the reference builds it).  Rules in oracle/quadtree_ref.py; built by sgb_quadtree.cu with one device->host read
+    (the tile count).
+
+    ``tiles``: [P, 4] fp64 boxes (xmin, ymin, xmax, ymax) in Morton order; ``labels``: int32 tile of every input point
+    (a dict when ``positions`` is); ``counts``: int32 points per tile; ``label(points)``: the tile of other points."""
+
+    def __init__(self, positions, max_tile_size: int = 50_000, max_depth: int = 15):
+        if not 1 <= int(max_depth) <= 15:
+            raise ValueError(f"max_depth must be in 1..15, got {max_depth}")
+        if int(max_tile_size) < 1:
+            raise ValueError(f"max_tile_size must be >= 1, got {max_tile_size}")
+        self.max_tile_size, self.max_depth = int(max_tile_size), int(max_depth)
+        named = isinstance(positions, dict)
+        parts = {k: _pos_arg(v) for k, v in positions.items()} if named else {None: _pos_arg(positions)}
+        if not parts:
+            raise ValueError("QuadTreeTiling: no positions")
+        dtypes = {p.dtype for p in parts.values()}
+        dt = torch.float64 if len(dtypes) > 1 else dtypes.pop()               # widening to fp64 is exact
+        pos = torch.cat([p.to(dt) for p in parts.values()]) if len(parts) > 1 else next(iter(parts.values()))
+        n, dev = pos.size(0), pos.device
+        lib = _lib.load()
+        cap = max(1, int(lib.sgb_quadtree_max_leaves(n, self.max_tile_size, self.max_depth)))
+        labels = _i32(n, dev)
+        self.root = torch.empty(3, dtype=torch.float64, device=dev)           # (xmin, ymin, scale)
+        meta = torch.empty(cap, 3, dtype=torch.int32, device=dev)
+        boxes = torch.empty(cap, 4, dtype=torch.float64, device=dev)
+        n_leaves = torch.zeros(1, dtype=torch.int32, device=dev)
+        ws = ops._ws(lib.sgb_quadtree_workspace_bytes(n, self.max_tile_size, self.max_depth), dev)
+        check(lib.sgb_quadtree_build(ptr(pos), int(pos.dtype == torch.float64), n, self.max_tile_size, self.max_depth,
+                                     ptr(labels), ptr(self.root), ptr(meta), ptr(boxes), cap, ptr(n_leaves), ptr(ws), ws.numel(),
+                                     stream_ptr(dev)), "quadtree_build")
+        ops._count(6 + self.max_depth + 12)                                   # + the radix sort's and the scan's launches
+        P = int(n_leaves.item())                                              # the one read-back
+        self._meta = meta[:P]
+        self.tiles = boxes[:P]
+        self.counts = self._meta[:, 2]
+        if named:
+            self.labels, o = {}, 0
+            for k, p in parts.items():
+                self.labels[k] = labels[o:o + p.size(0)]
+                o += p.size(0)
+        else:
+            self.labels = labels
+
+    def __len__(self) -> int:
+        return self.tiles.size(0)
+
+    @property
+    def levels(self) -> Tensor:
+        return self._meta[:, 1]
+
+    def label(self, points: Tensor) -> Tensor:
+        """int32 tile of each point: the leaf containing its cell (points outside the root clamp to the rim cells);
+        -1 for a cell of an empty quadrant."""
+        pts = _pos_arg(points)
+        out = _i32(pts.size(0), pts.device)
+        check(_lib.load().sgb_quadtree_label(ptr(pts), int(pts.dtype == torch.float64), pts.size(0), ptr(self.root), self.max_depth,
+                                             ptr(self._meta), len(self), ptr(out), stream_ptr(pts.device)), "quadtree_label")
+        ops._count(1)
+        return out
+
+    def fit_labels_and_masks(self, data: HeteroBatch, margin: float) -> Tuple[Dict[str, Tensor], Dict[str, Tensor]]:
+        """``TileFitDataset``: per node type the tile label (``TilePartition(data, labels, len(self))``) and the training
+        ``mask`` ``LitISTEncoder.get_losses`` reads = inside the own tile shrunk by the tile's margin (halved until the
+        shrunk tile is non-empty).  Nodes whose cell lies in an empty quadrant get label -1 and mask False."""
+        lib = _lib.load()
+        margins = fit_margins(self.tiles, margin)
+        labels, masks = {}, {}
+        for nt in data.node_types:
+            pos = _pos_arg(data[nt]["pos"])
+            lab = self.label(pos)
+            mask = torch.empty(pos.size(0), dtype=torch.bool, device=pos.device)
+            check(lib.sgb_quadtree_fit_mask(ptr(pos), int(pos.dtype == torch.float64), pos.size(0), ptr(lab), ptr(self.tiles),
+                                            ptr(margins), len(self), ptr(mask.view(torch.uint8)), stream_ptr(pos.device)),
+                  "quadtree_fit_mask")
+            ops._count(1)
+            labels[nt], masks[nt] = lab, mask
+        return labels, masks
+
+
+# ---------------------------------------------------------------------------------------------------------------------
 # training tiles: partition once, slice / collate per batch
 # ---------------------------------------------------------------------------------------------------------------------
 class TilePartition:
@@ -313,6 +418,20 @@ class TilePartition:
 # ---------------------------------------------------------------------------------------------------------------------
 # prediction tiles: tile + halo subgraph
 # ---------------------------------------------------------------------------------------------------------------------
+_MAX_CUT_RANGES = 1024            # candidate ranges of one cut (kMaxRanges of sgb_tilecut.cu)
+
+
+def _merge_spans(spans: Sequence[Tuple[int, int]], budget: int) -> List[Tuple[int, int]]:
+    """At most ``budget`` ranges covering ``spans`` (sorted, disjoint): the narrowest gaps are bridged.  The extra
+    candidates are dropped by the exact box test of the cut kernels."""
+    out = [list(r) for r in spans]
+    while len(out) > max(1, budget):
+        k = min(range(len(out) - 1), key=lambda i: out[i + 1][0] - out[i][1])
+        out[k][1] = out[k + 1][1]
+        del out[k + 1]
+    return [tuple(r) for r in out]
+
+
 class TilePredictSet:
     """``TilePredictDataset`` for a ``HeteroBatch`` on the GPU.  ``tiles``: [P, 4] (xmin, ymin, xmax, ymax) boxes;
     ``self[i]`` = the subgraph of the nodes inside box i grown by ``margin`` (half-open, tile_dataset.py:233-238) with
@@ -321,17 +440,27 @@ class TilePredictSet:
     The reference scans every node and every edge of the dataset for every tile.  When the boxes form a regular
     ``grid = (nx, ny)`` (``square_tiles``) and the margin is smaller than a tile, an index built once (nodes sorted by
     grid cell, edges by the cell of their source -- two stable radix sorts per type) restricts a tile's scan to the
-    3 x 3 neighbourhood of cells; the result is identical (same nodes, same order, same edges)."""
+    3 x 3 neighbourhood of cells; the result is identical (same nodes, same order, same edges).
+
+    ``tiles`` may also be a ``QuadTreeTiling``: the tiles are its leaves, and the index is built over the leaves (nodes
+    stably sorted by leaf, edges by the leaf of their source).  A tile's candidates are the leaves whose box meets its
+    margin-grown box (fp64, padded: a superset by construction), merged into ranges of adjacent leaf ids; the exact test
+    stays in the cut kernels, so any margin works and the result is again identical to ``subset``."""
 
     def __init__(self, data: HeteroBatch, tiles, margin: float = 0.0, grid: Optional[Tuple[int, int]] = None):
         self.data = data
+        tiling = tiles if isinstance(tiles, QuadTreeTiling) else None
+        if tiling is not None:
+            tiles = tiling.tiles
         self.tiles = [tuple(float(v) for v in t) for t in (tiles.tolist() if hasattr(tiles, "tolist") else tiles)]
         self.margin = float(margin)
         missing = [nt for nt in data.node_types if "pos" not in data[nt]]
         if missing:
             raise ValueError(f"Missing 'pos' attribute for node type: {', '.join(missing)}")
         self._index = None
-        if grid is not None and len(self.tiles) == grid[0] * grid[1] and len(self.tiles) > 1:
+        if tiling is not None:
+            self._build_leaf_index(tiling)
+        elif grid is not None and len(self.tiles) == grid[0] * grid[1] and len(self.tiles) > 1:
             self._build_index(grid)
 
     # -- coarse index ------------------------------------------------------------------------------------------------
@@ -370,7 +499,62 @@ class TilePredictSet:
             edge_ptr[et] = flat[o:o + P + 1]; o += P + 1
         self._index = dict(nx=nx, ny=ny, node_perm=node_perm, node_ptr=node_ptr, edge_perm=edge_perm, edge_ptr=edge_ptr, maps=maps)
 
+    def _build_leaf_index(self, tiling: "QuadTreeTiling") -> None:
+        P = len(self.tiles)
+        bucket = P                        # nodes in no leaf (an empty quadrant): a candidate of every tile
+        labels, node_perm, node_ptr, maps, ptrs = {}, {}, {}, {}, []
+        for nt in self.data.node_types:
+            pos = self.data[nt]["pos"]
+            lab = tiling.label(pos)
+            lab = torch.where(lab < 0, torch.full_like(lab, bucket), lab)
+            perm, indptr, _ = stable_argsort(lab, P + 1)
+            labels[nt], node_perm[nt] = lab, perm
+            ptrs.append(indptr)
+            maps[nt] = torch.full((pos.size(0),), -1, dtype=torch.int32, device=pos.device)
+        edge_perm = {}
+        for et in self.data.edge_types:
+            ei = self.data[et]["edge_index"]
+            perm, indptr, _ = stable_argsort(labels[et[0]].index_select(0, ei[0].long()), P + 1)
+            edge_perm[et] = perm
+            ptrs.append(indptr)
+        flat = torch.cat([p.to(torch.int64) for p in ptrs]).tolist() if ptrs else []
+        o = 0
+        for nt in self.data.node_types:
+            node_ptr[nt] = flat[o:o + P + 2]; o += P + 2
+        edge_ptr = {}
+        for et in self.data.edge_types:
+            edge_ptr[et] = flat[o:o + P + 2]; o += P + 2
+        # candidate leaves of every tile: leaf box (rim leaves open towards the outside: points beyond the root are
+        # labelled with rim leaves) meets the tile's margin-grown box, padded by more than an fp32 rounding of the bounds
+        b = tiling.tiles.detach().to("cpu", torch.float64)
+        lo = b.min(0).values
+        hi = b.max(0).values
+        inf = float("inf")
+        lb = b.clone()
+        lb[:, 0][b[:, 0] <= lo[0]] = -inf
+        lb[:, 1][b[:, 1] <= lo[1]] = -inf
+        lb[:, 2][b[:, 2] >= hi[2]] = inf
+        lb[:, 3][b[:, 3] >= hi[3]] = inf
+        m = self.margin
+        spans = []
+        for t in range(P):
+            x0, y0, x1, y1 = self.tiles[t]
+            ob = torch.tensor([x0 - m, y0 - m, x1 + m, y1 + m], dtype=torch.float64)
+            pad = 1e-6 * max(1.0, float(ob.abs().max()))
+            hit = ((lb[:, 0] <= ob[2] + pad) & (lb[:, 2] >= ob[0] - pad) & (lb[:, 1] <= ob[3] + pad) & (lb[:, 3] >= ob[1] - pad))
+            ids = hit.nonzero().flatten().tolist() + [bucket]
+            rng = []
+            for i in ids:
+                if rng and rng[-1][1] == i:
+                    rng[-1][1] = i + 1
+                else:
+                    rng.append([i, i + 1])
+            spans.append([tuple(r) for r in rng])
+        self._index = dict(spans=spans, node_perm=node_perm, node_ptr=node_ptr, edge_perm=edge_perm, edge_ptr=edge_ptr, maps=maps)
+
     def _neighbourhood(self, t: int) -> List[int]:
+        if "spans" in self._index:
+            return [c for a, b in self._index["spans"][t] for c in range(a, b)]
         nx, ny = self._index["nx"], self._index["ny"]
         i, j = t % nx, t // nx
         return [jj * nx + ii for jj in range(max(0, j - 1), min(ny, j + 2)) for ii in range(max(0, i - 1), min(nx, i + 2))]
@@ -471,16 +655,25 @@ class TilePredictSet:
     # -- several tiles at once --------------------------------------------------------------------------------------------
     def _slot_ranges(self, perm_ptr: List[int], tile_ids: Sequence[int], device):
         """Candidates of every slot as contiguous ranges of a cell-sorted id array: the 3 x 3 neighbourhood of a tile is
-        one range per grid row.  -> (start [R], off [R + 1], slot [R]) device arrays, R, total candidates."""
-        nx, ny = self._index["nx"], self._index["ny"]
+        one range per grid row; with the leaf index, one range per run of adjacent candidate leaves.
+        -> (start [R], off [R + 1], slot [R]) device arrays, R, total candidates."""
         start, length, slot = [], [], []
-        for s_, t in enumerate(tile_ids):
-            i, j = t % nx, t // nx
-            for jj in range(max(0, j - 1), min(ny, j + 2)):
-                c0, c1 = jj * nx + max(0, i - 1), jj * nx + min(nx, i + 2)
-                a, b = perm_ptr[c0], perm_ptr[c1]
-                if b > a:
-                    start.append(a); length.append(b - a); slot.append(s_)
+        if "spans" in self._index:
+            budget = _MAX_CUT_RANGES // len(tile_ids)
+            for s_, t in enumerate(tile_ids):
+                for c0, c1 in _merge_spans(self._index["spans"][t], budget):
+                    a, b = perm_ptr[c0], perm_ptr[c1]
+                    if b > a:
+                        start.append(a); length.append(b - a); slot.append(s_)
+        else:
+            nx, ny = self._index["nx"], self._index["ny"]
+            for s_, t in enumerate(tile_ids):
+                i, j = t % nx, t // nx
+                for jj in range(max(0, j - 1), min(ny, j + 2)):
+                    c0, c1 = jj * nx + max(0, i - 1), jj * nx + min(nx, i + 2)
+                    a, b = perm_ptr[c0], perm_ptr[c1]
+                    if b > a:
+                        start.append(a); length.append(b - a); slot.append(s_)
         off = [0]
         for n in length:
             off.append(off[-1] + n)
@@ -494,7 +687,8 @@ class TilePredictSet:
         and two device->host reads of the kept counts for the whole group (instead of ~100 launches and one read per
         tile).  Also returns ``info`` = per-slot node / edge counts (host lists) for batching by edge count."""
         if self._index is None:
-            raise RuntimeError("TilePredictSet.cut needs the grid index (pass grid=(nx, ny) with margin < tile size)")
+            raise RuntimeError("TilePredictSet.cut needs an index: tiles from a QuadTreeTiling, or grid=(nx, ny) with margin "
+                               "< tile size")
         tile_ids = [int(t) for t in tile_ids]
         T = len(tile_ids)
         if T == 0:
