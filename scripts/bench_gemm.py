@@ -4,7 +4,9 @@
 
 For every (op, M, N, K): ms per launch (CUDA events, 256 MB L2 flush between launches), effective fp32
 TFLOP/s (2MNK / t), achieved GB/s on the compulsory operand traffic, and the error against float64 on a
-65k-row sample: max |err| / max |ref| and the mean SIGNED relative error (the round-toward-zero bias)."""
+65k-row sample: max |err| / max |ref| and the mean SIGNED relative error (the round-toward-zero bias).
+`gather` is the gene-table forward of ISTEncoder's first projection (y = x w^T + b + table[ids], WM = 1 epilogue).
+SEGGER_B200_LIB=<path> times another build of libsegger_b200.so (A/B of two builds: run once per build, alternating)."""
 import argparse
 import json
 import os
@@ -20,7 +22,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--rows", type=int, default=1_000_000)
     ap.add_argument("--reps", type=int, default=5)
-    ap.add_argument("--only", default="", help="comma list of ops to run (fwd, dgrad, wgrad); default all")
+    ap.add_argument("--only", default="", help="comma list of ops to run (fwd, gather, dgrad, wgrad); default all")
     a = ap.parse_args()
     dev = torch.device("cuda", 0)
     R = a.rows
@@ -39,7 +41,7 @@ def main():
         return tot / a.reps * 1e-3
 
     rows = []
-    shapes = [("fwd", R, 384, 256), ("fwd", R, 384, 128), ("fwd", 2 * R, 64, 256), ("fwd", 2 * R, 64, 64), ("fwd", R, 64, 128),
+    shapes = [("gather", R, 384, 128), ("fwd", R, 384, 256), ("fwd", R, 384, 128), ("fwd", 2 * R, 64, 256), ("fwd", 2 * R, 64, 64), ("fwd", R, 64, 128),
               ("dgrad", R, 384, 256), ("dgrad", R, 384, 128), ("dgrad", R, 64, 128), ("dgrad", 2 * R, 64, 64),
               ("wgrad", R, 384, 256), ("wgrad", R, 384, 128), ("wgrad", 2 * R, 64, 256), ("wgrad", R, 64, 128),
               ("wgrad", 2 * R, 64, 64), ("wgrad", R, 256, 128)]
@@ -60,6 +62,18 @@ def main():
                 bias = float((((y.double() - ref) / ref)[m] * torch.sign(ref[m])).mean())
                 rows.append(dict(op=f"fwd exact={exact}", M=M, N=N, K=K, ms=t * 1e3, tflops=2 * M * N * K / t / 1e12,
                                  gbs=4 * (M * K + M * N) / t / 1e9, err=err, signed_bias=bias))
+        elif op == "gather":
+            n_genes = 500
+            x = torch.nn.functional.gelu(torch.randn(M, K, device=dev, generator=g))
+            w = torch.randn(N, K, device=dev, generator=g) / K ** 0.5
+            b = torch.randn(N, device=dev, generator=g)
+            table = torch.randn(n_genes, N, device=dev, generator=g)
+            ids = torch.randint(0, n_genes, (M,), device=dev, generator=g)
+            t = time_it(lambda: ops.linear_fwd(x, w, b, exact=0, gather=(ids, table)))
+            y, _ = ops.linear_fwd(x[:S], w, b, exact=0, gather=(ids[:S], table))
+            ref = x[:S].double() @ w.double().t() + b.double() + table.double()[ids[:S]]
+            rows.append(dict(op="gather", M=M, N=N, K=K, ms=t * 1e3, tflops=2 * M * N * K / t / 1e12,
+                             gbs=4 * (M * K + M * N) / t / 1e9, err=float((y.double() - ref).abs().max() / ref.abs().max())))
         elif op == "dgrad":
             dy = torch.randn(M, N, device=dev, generator=g)
             w = torch.randn(N, K, device=dev, generator=g) / K ** 0.5

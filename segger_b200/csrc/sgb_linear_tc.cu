@@ -1193,12 +1193,14 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_tf32x3_ts_kernel(const TcPar
         const int c0 = pass * PW;
         if (tc_dbg(p) & 8) break;
         // WM = 1 (this instantiation only gathers): the pass's table chunks are requested before the register -> staging
-        // copy so their L2 latency overlaps it
+        // copy so their L2 latency overlaps it.  Columns at or past N are not read: in the tail n-tile they would lie
+        // past the end of a table row (past the table itself for its last row when ld_gtab == N).
         float4 pre[WM == 1 ? LR : 1];
         if constexpr (WM == 1) {
+          const bool col_in = n0 + c0 + c4 < p.N;
 #pragma unroll
           for (int it = 0; it < LR; ++it)
-            pre[it] = fast_trow[it] != nullptr ? ldg4(fast_trow[it] + c0) : make_float4(0.f, 0.f, 0.f, 0.f);
+            pre[it] = (col_in && fast_trow[it] != nullptr) ? ldg4(fast_trow[it] + c0) : make_float4(0.f, 0.f, 0.f, 0.f);
         }
         __syncwarp();
 #pragma unroll
