@@ -660,10 +660,10 @@ def gatv2_bwd(x_l: Tensor, x_r: Tensor, att: Tensor, bias: Optional[Tensor], out
     lib = _lib.load()
     ws = _ws(lib.sgb_gatv2_bwd_workspace_bytes(n_dst, csr.E, H, C), dev)
     att, bias = _vec(att.reshape(-1)), _vec(bias)
-    # one virtual source per edge: the dst pass writes grad_x_l itself (NULL transposed CSR) where the sub-warp kernels apply
-    direct = (csr.one_source_per_edge and n_dst > 0 and csr.E > 0 and bool(lib.sgb_gatv2_quad_supported(H, C))
-              and os.environ.get("SEGGER_B200_GAT") != "legacy" and os.environ.get("SEGGER_B200_GAT_DIRECT", "1") != "0"
-              and all(t.data_ptr() % 16 == 0 and _ld(t) % 4 == 0 for t in (x_l, x_r, out_pre, grad_out, grad_x_l, grad_x_r)))
+    # one virtual source per edge: the dst pass writes grad_x_l itself (NULL transposed CSR) where the sub-warp kernels
+    # apply -- the library's whole rule, slope included: elsewhere it needs the transposed pass
+    direct = (csr.one_source_per_edge and n_dst > 0 and csr.E > 0 and os.environ.get("SEGGER_B200_GAT_DIRECT", "1") != "0"
+              and _quad_path(H, C, slope, x_l, x_r, att, bias, out_pre, grad_out, g_buf, grad_x_l, grad_x_r))
     t_rowptr, t_dst, t_pos = (None, None, None) if direct else (csr.t_rowptr, csr.t_dst, csr.t_pos)
     seed_val, seed_dev = _split_seed(seed)
     if e_logit is not None and (n_dst == 0 or tuple(e_logit.shape) != (csr.E, H) or not e_logit.is_contiguous() or not
