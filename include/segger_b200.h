@@ -1,7 +1,7 @@
 /*
  * libsegger_b200 -- C ABI of the B200-native segger hot path.
  *
- * Every entry point (73) is `extern "C"`, takes plain device pointers and sizes (no torch types),
+ * Every entry point (76) is `extern "C"`, takes plain device pointers and sizes (no torch types),
  * enqueues its work on the `stream` passed in (a cudaStream_t) and returns 0 on success or a
  * negative SGB_ERR_* code; the message is available from sgb_last_error() (thread-local).
  * The library never allocates, frees or retains device memory: outputs and workspaces are
@@ -327,6 +327,22 @@ SGB_API size_t sgb_pip_fill_scratch_bytes(int64_t E);
 SGB_API int sgb_pip_fill(const double* verts, const int64_t* ring_off, int64_t n_points, int64_t n_poly, double xmin, double ymin,
                  double cell, int nx, int ny, int64_t E, int32_t* edge_index, int64_t ld, void* ws, size_t ws_bytes,
                  void* scratch, size_t scratch_bytes, void* stream);
+/* Buffered outlines (data/utils/neighbors.py:229-231, geopandas .buffer(sqrt(area / pi) * buffer_ratio) then the join):
+ * per-ring area (signed shoelace, fp64, x relative to the first vertex), area-weighted centroid [n_poly,2] (triangle
+ * fan from the first vertex), box [n_poly,4] = (xmin, ymin, xmax, ymax) and dist = sqrt(|area| / pi) * ratio; each
+ * output may be NULL.  Fixed operation order, so a numpy evaluation gives the same doubles. */
+SGB_API int sgb_polygon_props(const double* verts, const int64_t* ring_off, int64_t n_poly, double ratio, double* area,
+                      double* centroid, double* box, double* dist, void* stream);
+/* neighbors.py:229-231: the join of sgb_pip_count / sgb_pip_fill (same workspace and scratch sizes, same output) against
+ * every ring grown by dist[poly] (device fp64): d > 0 keeps points inside the ring or at squared distance < d^2 from it
+ * (the exact Minkowski sum with a disc), d < 0 keeps points inside and at squared distance > d^2, d == 0 is the plain
+ * test.  The grid must cover the union of the polygon boxes grown by |d| (1 + 2^-20). */
+SGB_API int sgb_pip_buffered_count(const void* points, int points_f64, int64_t n_points, const double* verts,
+                      const int64_t* ring_off, const double* dist, int64_t n_poly, double xmin, double ymin, double cell,
+                      int nx, int ny, int32_t* total, void* ws, size_t ws_bytes, void* stream);
+SGB_API int sgb_pip_buffered_fill(const double* verts, const int64_t* ring_off, const double* dist, int64_t n_points,
+                      int64_t n_poly, double xmin, double ymin, double cell, int nx, int ny, int64_t E, int32_t* edge_index,
+                      int64_t ld, void* ws, size_t ws_bytes, void* scratch, size_t scratch_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Device-side tile slicing and batch assembly (SURVEY 8f rows N2/N3) and the masked compaction that ends

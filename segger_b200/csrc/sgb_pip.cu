@@ -4,7 +4,10 @@
 // Replaces cuspatial.quadtree_point_in_polygon behind
 //   points_in_polygons(..., predicate='contains')   /root/reference/src/segger/geometry/query.py:21-100
 //   setup_prediction_graph (shape modes)            /root/reference/src/segger/data/utils/neighbors.py:226-238
-// (the polygon buffering itself, geopandas .buffer at neighbors.py:229-230, is host geometry in the reference too).
+// The buffered variant (sgb_pip_buffered_count / _fill) takes the raw outlines plus one distance per ring and decides
+// membership in the exact Minkowski sum of the ring with a disc (or its erosion for a negative distance) instead of
+// asking geopandas .buffer (neighbors.py:229-231) for a grown polygon; sgb_polygon_props supplies the ring areas
+// those distances are derived from.
 //
 // Layout: points are binned into a uniform grid over the polygons' bounding box (cell ~ a polygon's extent) and
 // radix-sorted by cell (stable), so a polygon's bounding box covers a few contiguous ranges of the sorted point
@@ -67,13 +70,40 @@ __device__ __forceinline__ bool pip_inside(const double2* __restrict__ v, int nv
   return in;
 }
 
+// Squared distance from p to the ring: minimum over the edges a -> b of the point-to-segment distance, with
+//   dx, dy = b - a;  ex, ey = p - a;  L = dx^2 + dy^2;  t = L > 0 ? clamp((ex dx + ey dy) / L, 0, 1) : 0
+//   d2 = (ex - t dx)^2 + (ey - t dy)^2.
+// Every operation is rounded explicitly in this order (the oracle evaluates the same text in numpy).  The loop stops
+// early once the comparison with dd is decided: d2 < dd when `below`, d2 <= dd otherwise; the decision, not the
+// returned value, is the contract.
+__device__ __forceinline__ bool pip_ring_dist2_below(const double2* __restrict__ v, int nv, double px, double py, double dd,
+                                                     bool strict) {
+  double2 a = v[nv - 1];
+  for (int e = 0; e < nv; ++e) {
+    const double2 b = v[e];
+    const double dx = __dsub_rn(b.x, a.x), dy = __dsub_rn(b.y, a.y);
+    const double ex = __dsub_rn(px, a.x), ey = __dsub_rn(py, a.y);
+    const double L = __dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy));
+    double t = 0.0;
+    if (L > 0.0) t = fmin(fmax(__ddiv_rn(__dadd_rn(__dmul_rn(ex, dx), __dmul_rn(ey, dy)), L), 0.0), 1.0);
+    const double qx = __dsub_rn(ex, __dmul_rn(t, dx)), qy = __dsub_rn(ey, __dmul_rn(t, dy));
+    const double d2 = __dadd_rn(__dmul_rn(qx, qx), __dmul_rn(qy, qy));
+    if (strict ? d2 < dd : d2 <= dd) return true;
+    a = b;
+  }
+  return false;
+}
+
 // FILL == false: counts[poly] = number of points strictly inside;  FILL == true: writes (point, poly) at offsets[poly] + i
-template <bool FILL>
+// BUF == true: ring `poly` is grown by dist[poly] (d > 0: inside or squared distance < d^2; d < 0: inside and squared
+// distance > d^2; d == 0: inside); its box, and so the candidate range, grows by |d| (1 + 2^-20).  BUF == false is the
+// plain join and compiles to the same code as before the buffered variant existed.
+template <bool FILL, bool BUF>
 __global__ void __launch_bounds__(kPipThreads)
-pip_polygon_kernel(const double2* __restrict__ verts, const int64_t* __restrict__ ring_off, int64_t n_poly,
-                   const double2* __restrict__ sorted, const uint32_t* __restrict__ perm, const int32_t* __restrict__ cell_start,
-                   PipGrid g, int32_t* __restrict__ counts, const int32_t* __restrict__ offsets, uint32_t* __restrict__ out_point,
-                   uint32_t* __restrict__ out_poly) {
+pip_polygon_kernel(const double2* __restrict__ verts, const int64_t* __restrict__ ring_off, const double* __restrict__ dist,
+                   int64_t n_poly, const double2* __restrict__ sorted, const uint32_t* __restrict__ perm,
+                   const int32_t* __restrict__ cell_start, PipGrid g, int32_t* __restrict__ counts,
+                   const int32_t* __restrict__ offsets, uint32_t* __restrict__ out_point, uint32_t* __restrict__ out_poly) {
   __shared__ double2 sv[kPipMaxSmemVerts];
   __shared__ double sbox[4];
   __shared__ int scount;
@@ -105,9 +135,14 @@ pip_polygon_kernel(const double2* __restrict__ verts, const int64_t* __restrict_
     return;
   }
   const double2* v = in_smem ? sv : verts + v0;
-  int cx0 = pip_cell(sbox[0], g.xmin, g.inv_cell, g.nx), cx1 = pip_cell(sbox[2], g.xmin, g.inv_cell, g.nx);
-  int cy0 = pip_cell(sbox[1], g.ymin, g.inv_cell, g.ny), cy1 = pip_cell(sbox[3], g.ymin, g.inv_cell, g.ny);
-  // the grid covers the union of all polygon boxes, so the clamps only guard rounding at the upper edge
+  const double d = BUF ? dist[poly] : 0.0;
+  const double dd = __dmul_rn(d, d);
+  const double grow = BUF ? __dmul_rn(fabs(d), 1.0 + 0x1p-20) : 0.0;
+  const double bx0 = BUF ? __dsub_rn(sbox[0], grow) : sbox[0], by0 = BUF ? __dsub_rn(sbox[1], grow) : sbox[1];
+  const double bx1 = BUF ? __dadd_rn(sbox[2], grow) : sbox[2], by1 = BUF ? __dadd_rn(sbox[3], grow) : sbox[3];
+  int cx0 = pip_cell(bx0, g.xmin, g.inv_cell, g.nx), cx1 = pip_cell(bx1, g.xmin, g.inv_cell, g.nx);
+  int cy0 = pip_cell(by0, g.ymin, g.inv_cell, g.ny), cy1 = pip_cell(by1, g.ymin, g.inv_cell, g.ny);
+  // the grid covers the union of all (grown) polygon boxes, so the clamps only guard rounding at the upper edge
   cx0 = cx0 < 0 ? 0 : cx0; cy0 = cy0 < 0 ? 0 : cy0;
   cx1 = cx1 < 0 ? g.nx - 1 : cx1; cy1 = cy1 < 0 ? g.ny - 1 : cy1;
   const int base = FILL ? offsets[poly] : 0;
@@ -117,8 +152,18 @@ pip_polygon_kernel(const double2* __restrict__ verts, const int64_t* __restrict_
     const int end = cell_start[static_cast<int64_t>(cy) * g.nx + cx1 + 1];
     for (int s = beg + threadIdx.x; s < end; s += kPipThreads) {
       const double2 p = sorted[s];
-      if (p.x < sbox[0] || p.x > sbox[2] || p.y < sbox[1] || p.y > sbox[3]) continue;
-      if (pip_inside(v, nv, p.x, p.y)) {
+      bool hit;
+      if (BUF) {
+        if (p.x < bx0 || p.x > bx1 || p.y < by0 || p.y > by1) continue;
+        const bool inside = !(p.x < sbox[0] || p.x > sbox[2] || p.y < sbox[1] || p.y > sbox[3]) && pip_inside(v, nv, p.x, p.y);
+        if (d > 0.0) hit = inside || pip_ring_dist2_below(v, nv, p.x, p.y, dd, true);
+        else if (d < 0.0) hit = inside && !pip_ring_dist2_below(v, nv, p.x, p.y, dd, false);
+        else hit = inside;
+      } else {
+        if (p.x < sbox[0] || p.x > sbox[2] || p.y < sbox[1] || p.y > sbox[3]) continue;
+        hit = pip_inside(v, nv, p.x, p.y);
+      }
+      if (hit) {
         if (FILL) {
           const int slot = atomicAdd(&scount, 1);
           out_point[base + slot] = perm[s];
@@ -134,6 +179,61 @@ pip_polygon_kernel(const double2* __restrict__ verts, const int64_t* __restrict_
     __syncthreads();
     if (threadIdx.x == 0) counts[poly] = scount;
   }
+}
+
+// One thread per ring, sequential and in a fixed order (the oracle repeats it in numpy):
+//   area (signed, counter-clockwise > 0): x taken relative to the first vertex as GEOS's ring-area routine does,
+//     A = 0.5 * sum_{i=1..n-1} (x_i - x_0) * (y_{i+1} - y_{i-1}),  y_n = y_0;
+//   centroid: triangle fan from the first vertex, c_i = a_i x b_i with a_i = p_i - p_0, b_i = p_{i+1} - p_0,
+//     centroid = p_0 + sum c_i (a_i + b_i) / (3 sum c_i);  a ring whose fan area is 0 reports its first vertex;
+//   box: (xmin, ymin, xmax, ymax);  dist = sqrt(|A| / pi) * ratio.
+// An empty ring has area 0, a NaN centroid and the empty box (+inf, +inf, -inf, -inf).
+__global__ void polygon_props_kernel(const double2* __restrict__ verts, const int64_t* __restrict__ ring_off, int64_t n_poly,
+                                     double ratio, double* __restrict__ area, double2* __restrict__ centroid,
+                                     double4* __restrict__ box, double* __restrict__ dist) {
+  const int64_t r = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (r >= n_poly) return;
+  const double2* v = verts + ring_off[r];
+  int64_t n = ring_off[r + 1] - ring_off[r];
+  if (n >= 2 && v[0].x == v[n - 1].x && v[0].y == v[n - 1].y) --n;
+  double4 b = make_double4(INFINITY, INFINITY, -INFINITY, -INFINITY);
+  double s = 0.0, a2 = 0.0, sx = 0.0, sy = 0.0;
+  if (n > 0) {
+    const double2 p0 = v[0];
+    for (int64_t i = 0; i < n; ++i) {
+      const double2 p = v[i];
+      b.x = fmin(b.x, p.x); b.y = fmin(b.y, p.y); b.z = fmax(b.z, p.x); b.w = fmax(b.w, p.y);
+    }
+    if (n >= 3) {
+      for (int64_t i = 1; i < n; ++i) {
+        const double yn = v[i + 1 < n ? i + 1 : 0].y;
+        s = __dadd_rn(s, __dmul_rn(__dsub_rn(v[i].x, p0.x), __dsub_rn(yn, v[i - 1].y)));
+      }
+      for (int64_t i = 1; i + 1 < n; ++i) {
+        const double ax = __dsub_rn(v[i].x, p0.x), ay = __dsub_rn(v[i].y, p0.y);
+        const double bx = __dsub_rn(v[i + 1].x, p0.x), by = __dsub_rn(v[i + 1].y, p0.y);
+        const double c = __dsub_rn(__dmul_rn(ax, by), __dmul_rn(ay, bx));
+        a2 = __dadd_rn(a2, c);
+        sx = __dadd_rn(sx, __dmul_rn(c, __dadd_rn(ax, bx)));
+        sy = __dadd_rn(sy, __dmul_rn(c, __dadd_rn(ay, by)));
+      }
+    }
+  }
+  const double A = __dmul_rn(s, 0.5);
+  if (area) area[r] = A;
+  if (box) box[r] = b;
+  if (centroid) {
+    double2 c = make_double2(NAN, NAN);
+    if (n > 0) {
+      c = v[0];
+      if (a2 != 0.0) {
+        const double den = __dmul_rn(3.0, a2);
+        c = make_double2(__dadd_rn(c.x, __ddiv_rn(sx, den)), __dadd_rn(c.y, __ddiv_rn(sy, den)));
+      }
+    }
+    centroid[r] = c;
+  }
+  if (dist) dist[r] = __dmul_rn(__dsqrt_rn(__ddiv_rn(fabs(A), 3.141592653589793)), ratio);
 }
 
 __global__ void pip_emit_kernel(const uint32_t* __restrict__ point, const uint32_t* __restrict__ poly, int64_t E,
@@ -182,18 +282,22 @@ extern "C" size_t sgb_pip_workspace_bytes(int64_t n_points, int64_t n_poly, int 
   return pip_carve(nullptr, n_points, static_cast<int64_t>(nx) * ny, n_poly).total;
 }
 
-// Pass 1: bins the points, counts the contained points of every polygon, scans.  total[0] (device int32) = number of
-// (point, polygon) pairs; the caller reads it back to size the output of sgb_pip_fill (same workspace, untouched between).
-extern "C" int sgb_pip_count(const void* points, int points_f64, int64_t n_points, const double* verts, const int64_t* ring_off,
-                             int64_t n_poly, double xmin, double ymin, double cell, int nx, int ny, int32_t* total, void* ws,
-                             size_t ws_bytes, void* stream_) {
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+extern "C" size_t sgb_pip_fill_scratch_bytes(int64_t E) {
+  return 4 * align_up(static_cast<size_t>(E > 0 ? E : 1) * 4) + sort_pairs_workspace_bytes(E);
+}
+
+namespace sgb {
+namespace {
+
+int pip_count_impl(const char* what, const void* points, int points_f64, int64_t n_points, const double* verts,
+                   const int64_t* ring_off, const double* dist, int64_t n_poly, double xmin, double ymin, double cell, int nx,
+                   int ny, int32_t* total, void* ws, size_t ws_bytes, cudaStream_t stream) {
   SGB_REQUIRE(n_points >= 0 && n_points < (int64_t(1) << 31) && n_poly >= 0 && n_poly < (int64_t(1) << 31), SGB_ERR_RANGE,
-              "pip_count: size out of range");
-  SGB_REQUIRE(nx >= 1 && ny >= 1 && static_cast<int64_t>(nx) * ny < (int64_t(1) << 28) && cell > 0.0, SGB_ERR_ARG, "pip_count: bad grid");
-  SGB_REQUIRE(total && ws && (n_points == 0 || points) && (n_poly == 0 || (verts && ring_off)), SGB_ERR_ARG, "pip_count: null tensor");
-  SGB_REQUIRE(ws_bytes >= sgb_pip_workspace_bytes(n_points, n_poly, nx, ny), SGB_ERR_WORKSPACE, "pip_count: workspace too small");
-  if (n_points == 0 || n_poly == 0) { cudaMemsetAsync(total, 0, sizeof(int32_t), stream); return check_launch("pip_count(empty)"); }
+              "%s: size out of range", what);
+  SGB_REQUIRE(nx >= 1 && ny >= 1 && static_cast<int64_t>(nx) * ny < (int64_t(1) << 28) && cell > 0.0, SGB_ERR_ARG, "%s: bad grid", what);
+  SGB_REQUIRE(total && ws && (n_points == 0 || points) && (n_poly == 0 || (verts && ring_off)), SGB_ERR_ARG, "%s: null tensor", what);
+  SGB_REQUIRE(ws_bytes >= sgb_pip_workspace_bytes(n_points, n_poly, nx, ny), SGB_ERR_WORKSPACE, "%s: workspace too small", what);
+  if (n_points == 0 || n_poly == 0) { cudaMemsetAsync(total, 0, sizeof(int32_t), stream); return check_launch(what); }
   const int64_t ncell = static_cast<int64_t>(nx) * ny;
   PipWs w = pip_carve(ws, n_points, ncell, n_poly);
   const PipGrid g = make_grid(xmin, ymin, cell, nx, ny);
@@ -206,29 +310,28 @@ extern "C" int sgb_pip_count(const void* points, int points_f64, int64_t n_point
   if (rc != SGB_OK) return rc;
   if (points_f64) pip_gather_kernel<double><<<nb, 256, 0, stream>>>(static_cast<const double*>(points), w.perm, n_points, w.sorted);
   else pip_gather_kernel<float><<<nb, 256, 0, stream>>>(static_cast<const float*>(points), w.perm, n_points, w.sorted);
-  pip_polygon_kernel<false><<<static_cast<unsigned>(n_poly), kPipThreads, 0, stream>>>(
-      reinterpret_cast<const double2*>(verts), ring_off, n_poly, w.sorted, w.perm, w.cell_start, g, w.counts, nullptr, nullptr, nullptr);
+  if (dist)
+    pip_polygon_kernel<false, true><<<static_cast<unsigned>(n_poly), kPipThreads, 0, stream>>>(
+        reinterpret_cast<const double2*>(verts), ring_off, dist, n_poly, w.sorted, w.perm, w.cell_start, g, w.counts, nullptr,
+        nullptr, nullptr);
+  else
+    pip_polygon_kernel<false, false><<<static_cast<unsigned>(n_poly), kPipThreads, 0, stream>>>(
+        reinterpret_cast<const double2*>(verts), ring_off, nullptr, n_poly, w.sorted, w.perm, w.cell_start, g, w.counts, nullptr,
+        nullptr, nullptr);
   rc = exclusive_scan_i32(w.counts, w.offsets, n_poly, w.sort_ws, w.sort_bytes, stream);
   if (rc != SGB_OK) return rc;
   cudaMemcpyAsync(total, w.offsets + n_poly, sizeof(int32_t), cudaMemcpyDeviceToDevice, stream);
-  return check_launch("pip_count");
+  return check_launch(what);
 }
 
-// Pass 2: edge_index [2, E] int32 (row 0 = point index, row 1 = polygon index), point-major, polygon ascending.
-// scratch: 4 * E uint32 (pairs + sorted pairs) + sort workspace for E keys: sgb_pip_fill_scratch_bytes(E).
-extern "C" size_t sgb_pip_fill_scratch_bytes(int64_t E) {
-  return 4 * align_up(static_cast<size_t>(E > 0 ? E : 1) * 4) + sort_pairs_workspace_bytes(E);
-}
-
-extern "C" int sgb_pip_fill(const double* verts, const int64_t* ring_off, int64_t n_points, int64_t n_poly, double xmin, double ymin,
-                            double cell, int nx, int ny, int64_t E, int32_t* edge_index, int64_t ld, void* ws, size_t ws_bytes,
-                            void* scratch, size_t scratch_bytes, void* stream_) {
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  SGB_REQUIRE(E >= 0 && E < (int64_t(1) << 31), SGB_ERR_RANGE, "pip_fill: E out of range");
+int pip_fill_impl(const char* what, const double* verts, const int64_t* ring_off, const double* dist, int64_t n_points,
+                  int64_t n_poly, double xmin, double ymin, double cell, int nx, int ny, int64_t E, int32_t* edge_index, int64_t ld,
+                  void* ws, size_t ws_bytes, void* scratch, size_t scratch_bytes, cudaStream_t stream) {
+  SGB_REQUIRE(E >= 0 && E < (int64_t(1) << 31), SGB_ERR_RANGE, "%s: E out of range", what);
   if (E == 0) return SGB_OK;
-  SGB_REQUIRE(verts && ring_off && edge_index && ws && scratch && ld >= E, SGB_ERR_ARG, "pip_fill: null tensor");
-  SGB_REQUIRE(ws_bytes >= sgb_pip_workspace_bytes(n_points, n_poly, nx, ny), SGB_ERR_WORKSPACE, "pip_fill: workspace too small");
-  SGB_REQUIRE(scratch_bytes >= sgb_pip_fill_scratch_bytes(E), SGB_ERR_WORKSPACE, "pip_fill: scratch too small");
+  SGB_REQUIRE(verts && ring_off && edge_index && ws && scratch && ld >= E, SGB_ERR_ARG, "%s: null tensor", what);
+  SGB_REQUIRE(ws_bytes >= sgb_pip_workspace_bytes(n_points, n_poly, nx, ny), SGB_ERR_WORKSPACE, "%s: workspace too small", what);
+  SGB_REQUIRE(scratch_bytes >= sgb_pip_fill_scratch_bytes(E), SGB_ERR_WORKSPACE, "%s: scratch too small", what);
   const int64_t ncell = static_cast<int64_t>(nx) * ny;
   PipWs w = pip_carve(ws, n_points, ncell, n_poly);
   const PipGrid g = make_grid(xmin, ymin, cell, nx, ny);
@@ -238,12 +341,71 @@ extern "C" int sgb_pip_fill(const double* verts, const int64_t* ring_off, int64_
   uint32_t* pl = reinterpret_cast<uint32_t*>(p); p += eb;
   uint32_t* spt = reinterpret_cast<uint32_t*>(p); p += eb;
   uint32_t* spl = reinterpret_cast<uint32_t*>(p); p += eb;
-  pip_polygon_kernel<true><<<static_cast<unsigned>(n_poly), kPipThreads, 0, stream>>>(
-      reinterpret_cast<const double2*>(verts), ring_off, n_poly, w.sorted, w.perm, w.cell_start, g, nullptr, w.offsets, pt, pl);
+  if (dist)
+    pip_polygon_kernel<true, true><<<static_cast<unsigned>(n_poly), kPipThreads, 0, stream>>>(
+        reinterpret_cast<const double2*>(verts), ring_off, dist, n_poly, w.sorted, w.perm, w.cell_start, g, nullptr, w.offsets, pt, pl);
+  else
+    pip_polygon_kernel<true, false><<<static_cast<unsigned>(n_poly), kPipThreads, 0, stream>>>(
+        reinterpret_cast<const double2*>(verts), ring_off, nullptr, n_poly, w.sorted, w.perm, w.cell_start, g, nullptr, w.offsets, pt,
+        pl);
   // pairs are grouped by polygon (ascending) with arbitrary order inside a group; a stable sort by point id makes the
   // list point-major with polygons ascending per point -- independent of the order the atomics handed out slots
   int rc = sort_pairs(pt, pl, spt, spl, E, bits_for(n_points), p, sort_pairs_workspace_bytes(E), stream);
   if (rc != SGB_OK) return rc;
   pip_emit_kernel<<<static_cast<unsigned>(ceil_div(E, 256)), 256, 0, stream>>>(spt, spl, E, edge_index, ld);
-  return check_launch("pip_fill");
+  return check_launch(what);
+}
+
+}  // namespace
+}  // namespace sgb
+
+// Pass 1: bins the points, counts the contained points of every polygon, scans.  total[0] (device int32) = number of
+// (point, polygon) pairs; the caller reads it back to size the output of sgb_pip_fill (same workspace, untouched between).
+extern "C" int sgb_pip_count(const void* points, int points_f64, int64_t n_points, const double* verts, const int64_t* ring_off,
+                             int64_t n_poly, double xmin, double ymin, double cell, int nx, int ny, int32_t* total, void* ws,
+                             size_t ws_bytes, void* stream) {
+  return pip_count_impl("pip_count", points, points_f64, n_points, verts, ring_off, nullptr, n_poly, xmin, ymin, cell, nx, ny,
+                        total, ws, ws_bytes, static_cast<cudaStream_t>(stream));
+}
+
+// Pass 2: edge_index [2, E] int32 (row 0 = point index, row 1 = polygon index), point-major, polygon ascending.
+// scratch: 4 * E uint32 (pairs + sorted pairs) + sort workspace for E keys: sgb_pip_fill_scratch_bytes(E).
+extern "C" int sgb_pip_fill(const double* verts, const int64_t* ring_off, int64_t n_points, int64_t n_poly, double xmin, double ymin,
+                            double cell, int nx, int ny, int64_t E, int32_t* edge_index, int64_t ld, void* ws, size_t ws_bytes,
+                            void* scratch, size_t scratch_bytes, void* stream) {
+  return pip_fill_impl("pip_fill", verts, ring_off, nullptr, n_points, n_poly, xmin, ymin, cell, nx, ny, E, edge_index, ld, ws,
+                       ws_bytes, scratch, scratch_bytes, static_cast<cudaStream_t>(stream));
+}
+
+// The same two passes against rings grown by dist[poly] (device fp64, one per ring); the grid must cover the union of
+// the boxes grown by |dist| (1 + 2^-20).
+extern "C" int sgb_pip_buffered_count(const void* points, int points_f64, int64_t n_points, const double* verts,
+                                      const int64_t* ring_off, const double* dist, int64_t n_poly, double xmin, double ymin,
+                                      double cell, int nx, int ny, int32_t* total, void* ws, size_t ws_bytes, void* stream) {
+  SGB_REQUIRE(n_poly <= 0 || dist, SGB_ERR_ARG, "pip_buffered_count: null dist");
+  return pip_count_impl("pip_buffered_count", points, points_f64, n_points, verts, ring_off, dist, n_poly, xmin, ymin, cell, nx,
+                        ny, total, ws, ws_bytes, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int sgb_pip_buffered_fill(const double* verts, const int64_t* ring_off, const double* dist, int64_t n_points,
+                                     int64_t n_poly, double xmin, double ymin, double cell, int nx, int ny, int64_t E,
+                                     int32_t* edge_index, int64_t ld, void* ws, size_t ws_bytes, void* scratch,
+                                     size_t scratch_bytes, void* stream) {
+  SGB_REQUIRE(E == 0 || dist, SGB_ERR_ARG, "pip_buffered_fill: null dist");
+  return pip_fill_impl("pip_buffered_fill", verts, ring_off, dist, n_points, n_poly, xmin, ymin, cell, nx, ny, E, edge_index, ld,
+                       ws, ws_bytes, scratch, scratch_bytes, static_cast<cudaStream_t>(stream));
+}
+
+// Per-ring area / centroid / box and, when `dist` is given, the buffer distance sqrt(|area| / pi) * ratio.
+// area [n_poly], centroid [n_poly, 2], box [n_poly, 4] = (xmin, ymin, xmax, ymax), dist [n_poly]: fp64, each may be NULL.
+extern "C" int sgb_polygon_props(const double* verts, const int64_t* ring_off, int64_t n_poly, double ratio, double* area,
+                                 double* centroid, double* box, double* dist, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  SGB_REQUIRE(n_poly >= 0 && n_poly < (int64_t(1) << 31), SGB_ERR_RANGE, "polygon_props: size out of range");
+  if (n_poly == 0) return SGB_OK;
+  SGB_REQUIRE(verts && ring_off, SGB_ERR_ARG, "polygon_props: null tensor");
+  polygon_props_kernel<<<static_cast<unsigned>(ceil_div(n_poly, 128)), 128, 0, stream>>>(
+      reinterpret_cast<const double2*>(verts), ring_off, n_poly, ratio, area, reinterpret_cast<double2*>(centroid),
+      reinterpret_cast<double4*>(box), dist);
+  return check_launch("polygon_props");
 }

@@ -166,18 +166,25 @@ def setup_prediction_graph(tx, bd, max_k: int, buffer_ratio: float, mode: str = 
     ``mode`` 'cell' / 'nucleus': transcripts strictly inside the outlines of that boundary type, each grown by
     ``sqrt(area / pi) * buffer_ratio`` -- the point-in-polygon join runs on the GPU (``segger_b200.geometry``);
     returns int32 CPU ``[2, E]`` = (transcript row, boundary row) like the reference.  ``bd`` is either a
-    GeoDataFrame (buffered on the host with shapely exactly as the reference does, :229-231) or outlines that
-    are buffered already: a ``geometry.PackedPolygons`` or a ``(verts, ring_off)`` pair (``buffer_ratio`` must
-    then be 0 or None).
+    GeoDataFrame (buffered on the host with shapely exactly as the reference does, :229-231), raw outlines as a
+    ``geometry.Outlines`` (rings of the mode's ``boundary_type`` when it is given, renumbered from 0 as the
+    reference's ``reset_index(drop=True)`` does, then buffered on the GPU -- no geopandas or shapely needed), or
+    outlines that are buffered already: a ``geometry.PackedPolygons`` or a ``(verts, ring_off)`` pair
+    (``buffer_ratio`` must then be 0 or None).
     ``mode`` 'uniform': k nearest transcripts of every boundary centroid.  The reference calls
     ``kdtree_neighbors(points, query, max_k)`` without the mandatory ``max_dist`` there and raises TypeError
     (SURVEY Appendix B.4); the evident intent -- no radius cap -- is what this does.  ``bd`` may be the
-    GeoDataFrame or an [M, 2] centroid array; rows are (boundary row, transcript row) as that call returns them.
+    GeoDataFrame, an ``Outlines`` (centroids computed on the GPU) or an [M, 2] centroid array; rows are
+    (boundary row, transcript row) as that call returns them.
     """
-    from .geometry import PackedPolygons, pack_rings, points_in_polygons
+    from .geometry import Outlines, PackedPolygons, pack_rings, points_in_polygons
     points = _xy(tx)
     if mode == "uniform":
-        if hasattr(bd, "geometry"):
+        if isinstance(bd, Outlines):
+            query = bd.centroids(device)
+            if not np.isfinite(query).all():
+                raise ValueError("setup_prediction_graph: an empty outline has no centroid")
+        elif hasattr(bd, "geometry"):
             query = bd.geometry.centroid.get_coordinates().values
         else:
             query = bd.cpu().numpy() if isinstance(bd, Tensor) else np.asarray(bd)
@@ -188,7 +195,11 @@ def setup_prediction_graph(tx, bd, max_k: int, buffer_ratio: float, mode: str = 
         return edge_index.cpu()
     if mode not in ("cell", "nucleus"):
         raise ValueError(f"setup_prediction_graph: unknown mode '{mode}' (expected 'nucleus', 'cell' or 'uniform')")
-    if isinstance(bd, PackedPolygons):
+    if isinstance(bd, Outlines):
+        outlines = bd if bd.boundary_type is None else bd.of_type("cell" if mode == "cell" else "nucleus")
+        polys = outlines.buffered(buffer_ratio or 0.0, device)
+        buffer_ratio = 0
+    elif isinstance(bd, PackedPolygons):
         polys = bd
     elif isinstance(bd, (tuple, list)) and len(bd) == 2:
         polys = PackedPolygons(*bd)
@@ -200,8 +211,9 @@ def setup_prediction_graph(tx, bd, max_k: int, buffer_ratio: float, mode: str = 
         polys = PackedPolygons(*pack_rings([np.asarray(g.exterior.coords) for g in polygons]))
         buffer_ratio = 0
     else:
-        raise TypeError("setup_prediction_graph: `bd` must be a GeoDataFrame, a PackedPolygons or (verts, ring_off)")
+        raise TypeError("setup_prediction_graph: `bd` must be a GeoDataFrame, an Outlines, a PackedPolygons or "
+                        "(verts, ring_off)")
     if buffer_ratio:
         raise ValueError("setup_prediction_graph: packed outlines are taken as already buffered (pass buffer_ratio=0); "
-                         "buffering is host geometry (shapely), as in the reference")
+                         "pass raw outlines as a geometry.Outlines to buffer them on the GPU")
     return points_in_polygons(points, polys, device=device, device_output=False)
