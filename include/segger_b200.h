@@ -1,7 +1,7 @@
 /*
  * libsegger_b200 -- C ABI of the B200-native segger hot path.
  *
- * Every entry point (76) is `extern "C"`, takes plain device pointers and sizes (no torch types),
+ * Every entry point (79) is `extern "C"`, takes plain device pointers and sizes (no torch types),
  * enqueues its work on the `stream` passed in (a cudaStream_t) and returns 0 on success or a
  * negative SGB_ERR_* code; the message is available from sgb_last_error() (thread-local).
  * The library never allocates, frees or retains device memory: outputs and workspaces are
@@ -343,6 +343,29 @@ SGB_API int sgb_pip_buffered_count(const void* points, int points_f64, int64_t n
 SGB_API int sgb_pip_buffered_fill(const double* verts, const int64_t* ring_off, const double* dist, int64_t n_points,
                       int64_t n_poly, double xmin, double ymin, double cell, int nx, int ny, int64_t E, int32_t* edge_index,
                       int64_t ld, void* ws, size_t ws_bytes, void* scratch, size_t scratch_bytes, void* stream);
+/* Outlines with holes and several parts (the GeoArrow / cuSpatial polygon layout the reference's GeoSeries carries):
+ * ring_off [R+1] = vertices of ring r, part_off [Q+1] = rings of part q (the first its exterior, the rest its holes),
+ * geom_off [n_geom+1] = parts of geometry g (one boundary row, one polygon id of the output).  Per geometry: area =
+ * sum of |ring area| over exteriors minus holes, centroid = the area-weighted mean of the ring centroids, box = union
+ * of the ring boxes, dist = sqrt(|area| / pi) * ratio; a geometry of one ring gives |area| and the centroid, box and
+ * dist of sgb_polygon_props bit for bit.  Each output may be NULL. */
+SGB_API int sgb_polygon_props_multi(const double* verts, const int64_t* ring_off, const int64_t* part_off,
+                      const int64_t* geom_off, int64_t n_geom, double ratio, double* area, double* centroid, double* box,
+                      double* dist, void* stream);
+/* The join of sgb_pip_count / _fill (same grid, workspace, scratch and output, geometries in place of rings) against
+ * that layout: p is in geometry g iff the even-odd rule over all rings of g says so (the XOR of the single-ring
+ * decisions; for valid geometry the union of the parts minus their holes), listed once per geometry.  dist [n_geom]
+ * device fp64 or NULL (the plain join): geometry g grown by dist[g] as sgb_pip_buffered_count grows one ring, the
+ * distance taken to the nearest edge of any of its rings; the grid must cover the geometry boxes grown by
+ * |dist| (1 + 2^-20). */
+SGB_API int sgb_pip_multi_count(const void* points, int points_f64, int64_t n_points, const double* verts,
+                      const int64_t* ring_off, const int64_t* part_off, const int64_t* geom_off, const double* dist,
+                      int64_t n_geom, double xmin, double ymin, double cell, int nx, int ny, int32_t* total, void* ws,
+                      size_t ws_bytes, void* stream);
+SGB_API int sgb_pip_multi_fill(const double* verts, const int64_t* ring_off, const int64_t* part_off, const int64_t* geom_off,
+                      const double* dist, int64_t n_points, int64_t n_geom, double xmin, double ymin, double cell, int nx,
+                      int ny, int64_t E, int32_t* edge_index, int64_t ld, void* ws, size_t ws_bytes, void* scratch,
+                      size_t scratch_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Device-side tile slicing and batch assembly (SURVEY 8f rows N2/N3) and the masked compaction that ends

@@ -88,6 +88,11 @@ _PROTOS = {
                                        c_int, c_vp, c_vp, c_sz, c_vp]),
     "sgb_pip_buffered_fill": (c_int, [c_vp, c_vp, c_vp, c_i64, c_i64, C.c_double, C.c_double, C.c_double, c_int, c_int, c_i64,
                                       c_vp, c_i64, c_vp, c_sz, c_vp, c_sz, c_vp]),
+    "sgb_polygon_props_multi": (c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, C.c_double, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "sgb_pip_multi_count": (c_int, [c_vp, c_int, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, C.c_double, C.c_double, C.c_double,
+                                    c_int, c_int, c_vp, c_vp, c_sz, c_vp]),
+    "sgb_pip_multi_fill": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, C.c_double, C.c_double, C.c_double, c_int, c_int,
+                                   c_i64, c_vp, c_i64, c_vp, c_sz, c_vp, c_sz, c_vp]),
     "sgb_gatv2_quad_supported": (c_int, [c_int, c_int]),
     "sgb_l2norm_fwd": (c_int, [c_vp, c_i64, c_i64, c_int, c_f32, c_vp, c_i64, c_vp, c_vp]),
     "sgb_l2norm_bwd": (c_int, [c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_int, c_f32, c_vp, c_i64, c_vp]),

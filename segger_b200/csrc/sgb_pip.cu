@@ -7,7 +7,9 @@
 // The buffered variant (sgb_pip_buffered_count / _fill) takes the raw outlines plus one distance per ring and decides
 // membership in the exact Minkowski sum of the ring with a disc (or its erosion for a negative distance) instead of
 // asking geopandas .buffer (neighbors.py:229-231) for a grown polygon; sgb_polygon_props supplies the ring areas
-// those distances are derived from.
+// those distances are derived from.  Outlines with holes and several parts (sgb_pip_multi_count / _fill,
+// sgb_polygon_props_multi) come in the GeoArrow / cuSpatial layout (ring_off, part_off, geom_off): one CTA per
+// geometry, the even-odd rule over all of its rings.
 //
 // Layout: points are binned into a uniform grid over the polygons' bounding box (cell ~ a polygon's extent) and
 // radix-sorted by cell (stable), so a polygon's bounding box covers a few contiguous ranges of the sorted point
@@ -24,6 +26,7 @@ namespace {
 
 constexpr int kPipThreads = 128;
 constexpr int kPipMaxSmemVerts = 1024;          // rings longer than this are read from global memory
+constexpr int kPipMaxSmemRings = 64;            // multi-ring geometries: ring descriptors beyond this come from global
 
 struct PipGrid {
   double xmin, ymin, inv_cell;
@@ -94,45 +97,137 @@ __device__ __forceinline__ bool pip_ring_dist2_below(const double2* __restrict__
   return false;
 }
 
+// One ring of a multi-ring geometry: its first vertex relative to the geometry's first vertex, its vertex count
+// after dropping a closing duplicate, and its box (empty for rings of fewer than 3 vertices, which match nothing).
+struct PipRing {
+  double4 box;
+  int start, nv;
+};
+
+__device__ __forceinline__ PipRing pip_ring_info(const double2* __restrict__ verts, const int64_t* __restrict__ ring_off,
+                                                 int64_t r, int64_t v0) {
+  PipRing R;
+  const int64_t s = ring_off[r];
+  R.start = static_cast<int>(s - v0);
+  R.nv = static_cast<int>(ring_off[r + 1] - s);
+  if (R.nv >= 2) {
+    const double2 f = verts[s], l = verts[s + R.nv - 1];
+    if (f.x == l.x && f.y == l.y) --R.nv;
+  }
+  R.box = make_double4(INFINITY, INFINITY, -INFINITY, -INFINITY);
+  if (R.nv >= 3)
+    for (int i = 0; i < R.nv; ++i) {
+      const double2 p = verts[s + i];
+      R.box.x = fmin(R.box.x, p.x); R.box.y = fmin(R.box.y, p.y);
+      R.box.z = fmax(R.box.z, p.x); R.box.w = fmax(R.box.w, p.y);
+    }
+  return R;
+}
+
+// Ring i of the geometry: from shared memory for the first kPipMaxSmemRings rings, recomputed from global memory
+// beyond (an outline with that many holes or parts is rare).
+__device__ __forceinline__ PipRing pip_ring_at(const PipRing* __restrict__ sring, int i, const double2* __restrict__ verts,
+                                               const int64_t* __restrict__ ring_off, int64_t r0, int64_t v0) {
+  return i < kPipMaxSmemRings ? sring[i] : pip_ring_info(verts, ring_off, r0 + i, v0);
+}
+
+// Membership of p in a multi-ring geometry: inside = XOR over its rings of the single-ring decision (ring box, then the
+// even-odd test) -- the even-odd rule over all rings; with BUF the distance is the minimum over all rings, decided
+// ring by ring with the same early exit as one ring.
+template <bool BUF>
+__device__ __forceinline__ bool pip_multi_hit(const PipRing* __restrict__ sring, int nring, const double2* __restrict__ vbase,
+                                              const double2* __restrict__ verts, const int64_t* __restrict__ ring_off,
+                                              int64_t r0, int64_t v0, double px, double py, double d, double dd) {
+  bool inside = false;
+  for (int i = 0; i < nring; ++i) {
+    const PipRing R = pip_ring_at(sring, i, verts, ring_off, r0, v0);
+    if (R.nv < 3 || px < R.box.x || px > R.box.z || py < R.box.y || py > R.box.w) continue;
+    if (pip_inside(vbase + R.start, R.nv, px, py)) inside = !inside;
+  }
+  if (!BUF || d == 0.0) return inside;
+  if (d > 0.0 && inside) return true;
+  if (d < 0.0 && !inside) return false;
+  for (int i = 0; i < nring; ++i) {
+    const PipRing R = pip_ring_at(sring, i, verts, ring_off, r0, v0);
+    if (R.nv >= 3 && pip_ring_dist2_below(vbase + R.start, R.nv, px, py, dd, d > 0.0)) return d > 0.0;
+  }
+  return d < 0.0;
+}
+
 // FILL == false: counts[poly] = number of points strictly inside;  FILL == true: writes (point, poly) at offsets[poly] + i
 // BUF == true: ring `poly` is grown by dist[poly] (d > 0: inside or squared distance < d^2; d < 0: inside and squared
 // distance > d^2; d == 0: inside); its box, and so the candidate range, grows by |d| (1 + 2^-20).  BUF == false is the
 // plain join and compiles to the same code as before the buffered variant existed.
-template <bool FILL, bool BUF>
+// MULTI == true: `poly` is geometry g of the polygon layout (rings part_off[geom_off[g]] .. part_off[geom_off[g + 1]],
+// their vertices one contiguous range), tested with pip_multi_hit against the union of its ring boxes.  The geometry's
+// vertices are staged in shared memory while they total at most kPipMaxSmemVerts, the first kPipMaxSmemRings ring
+// descriptors always.  MULTI == false compiles to the same code as before the multi-ring variant existed.
+template <bool FILL, bool BUF, bool MULTI = false>
 __global__ void __launch_bounds__(kPipThreads)
 pip_polygon_kernel(const double2* __restrict__ verts, const int64_t* __restrict__ ring_off, const double* __restrict__ dist,
                    int64_t n_poly, const double2* __restrict__ sorted, const uint32_t* __restrict__ perm,
                    const int32_t* __restrict__ cell_start, PipGrid g, int32_t* __restrict__ counts,
-                   const int32_t* __restrict__ offsets, uint32_t* __restrict__ out_point, uint32_t* __restrict__ out_poly) {
+                   const int32_t* __restrict__ offsets, uint32_t* __restrict__ out_point, uint32_t* __restrict__ out_poly,
+                   const int64_t* __restrict__ part_off = nullptr, const int64_t* __restrict__ geom_off = nullptr) {
   __shared__ double2 sv[kPipMaxSmemVerts];
   __shared__ double sbox[4];
   __shared__ int scount;
+  __shared__ PipRing sring[MULTI ? kPipMaxSmemRings : 1];
   const int64_t poly = blockIdx.x;
   if (poly >= n_poly) return;
-  const int64_t v0 = ring_off[poly];
-  int nv = static_cast<int>(ring_off[poly + 1] - v0);
-  // a closed ring that repeats its first vertex at the end: drop the duplicate (zero-length edge)
-  if (nv >= 2) {
-    const double2 f = verts[v0], l = verts[v0 + nv - 1];
-    if (f.x == l.x && f.y == l.y) --nv;
+  int64_t v0, r0 = 0;
+  int nv, nring = 0;
+  if constexpr (MULTI) {
+    r0 = part_off[geom_off[poly]];
+    const int64_t r1 = part_off[geom_off[poly + 1]];
+    nring = static_cast<int>(r1 - r0);
+    v0 = ring_off[r0];
+    nv = static_cast<int>(ring_off[r1] - v0);
+  } else {
+    v0 = ring_off[poly];
+    nv = static_cast<int>(ring_off[poly + 1] - v0);
+    // a closed ring that repeats its first vertex at the end: drop the duplicate (zero-length edge)
+    if (nv >= 2) {
+      const double2 f = verts[v0], l = verts[v0 + nv - 1];
+      if (f.x == l.x && f.y == l.y) --nv;
+    }
   }
   const bool in_smem = nv <= kPipMaxSmemVerts;
   if (threadIdx.x == 0) { scount = 0; sbox[0] = INFINITY; sbox[1] = INFINITY; sbox[2] = -INFINITY; sbox[3] = -INFINITY; }
   __syncthreads();
   if (in_smem)
     for (int i = threadIdx.x; i < nv; i += kPipThreads) sv[i] = verts[v0 + i];
-  // bounding box: one thread (rings are tens of vertices)
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < nv; ++i) {
-      const double2 p = verts[v0 + i];
-      sbox[0] = fmin(sbox[0], p.x); sbox[1] = fmin(sbox[1], p.y);
-      sbox[2] = fmax(sbox[2], p.x); sbox[3] = fmax(sbox[3], p.y);
+  if constexpr (MULTI) {
+    const int nstage = nring < kPipMaxSmemRings ? nring : kPipMaxSmemRings;
+    for (int i = threadIdx.x; i < nstage; i += kPipThreads) sring[i] = pip_ring_info(verts, ring_off, r0 + i, v0);
+    __syncthreads();
+    // the geometry's box: the union of its ring boxes
+    if (threadIdx.x == 0) {
+      for (int i = 0; i < nring; ++i) {
+        const double4 b = pip_ring_at(sring, i, verts, ring_off, r0, v0).box;
+        sbox[0] = fmin(sbox[0], b.x); sbox[1] = fmin(sbox[1], b.y);
+        sbox[2] = fmax(sbox[2], b.z); sbox[3] = fmax(sbox[3], b.w);
+      }
     }
-  }
-  __syncthreads();
-  if (nv < 3) {
-    if (!FILL && threadIdx.x == 0) counts[poly] = 0;
-    return;
+    __syncthreads();
+    if (!(sbox[0] <= sbox[2])) {                        // no ring of 3 or more vertices: matches nothing
+      if (!FILL && threadIdx.x == 0) counts[poly] = 0;
+      return;
+    }
+  } else {
+    // bounding box: one thread (rings are tens of vertices)
+    if (threadIdx.x == 0) {
+      for (int i = 0; i < nv; ++i) {
+        const double2 p = verts[v0 + i];
+        sbox[0] = fmin(sbox[0], p.x); sbox[1] = fmin(sbox[1], p.y);
+        sbox[2] = fmax(sbox[2], p.x); sbox[3] = fmax(sbox[3], p.y);
+      }
+    }
+    __syncthreads();
+    if (nv < 3) {
+      if (!FILL && threadIdx.x == 0) counts[poly] = 0;
+      return;
+    }
   }
   const double2* v = in_smem ? sv : verts + v0;
   const double d = BUF ? dist[poly] : 0.0;
@@ -153,7 +248,10 @@ pip_polygon_kernel(const double2* __restrict__ verts, const int64_t* __restrict_
     for (int s = beg + threadIdx.x; s < end; s += kPipThreads) {
       const double2 p = sorted[s];
       bool hit;
-      if (BUF) {
+      if constexpr (MULTI) {
+        if (p.x < bx0 || p.x > bx1 || p.y < by0 || p.y > by1) continue;
+        hit = pip_multi_hit<BUF>(sring, nring, v, verts, ring_off, r0, v0, p.x, p.y, d, dd);
+      } else if (BUF) {
         if (p.x < bx0 || p.x > bx1 || p.y < by0 || p.y > by1) continue;
         const bool inside = !(p.x < sbox[0] || p.x > sbox[2] || p.y < sbox[1] || p.y > sbox[3]) && pip_inside(v, nv, p.x, p.y);
         if (d > 0.0) hit = inside || pip_ring_dist2_below(v, nv, p.x, p.y, dd, true);
@@ -236,6 +334,81 @@ __global__ void polygon_props_kernel(const double2* __restrict__ verts, const in
   if (dist) dist[r] = __dmul_rn(__dsqrt_rn(__ddiv_rn(fabs(A), 3.141592653589793)), ratio);
 }
 
+// One ring of polygon_props_kernel, in its operation order: signed area A, fan centroid c (the first vertex when the fan
+// area is 0), box; returns the vertex count after dropping a closing duplicate (0: A = 0 and the box empty, c
+// untouched).  polygon_props_kernel keeps its own copy of these lines so that its code stays what it was.
+__device__ __forceinline__ int64_t ring_props(const double2* __restrict__ v, int64_t n, double& A, double2& c, double4& b) {
+  if (n >= 2 && v[0].x == v[n - 1].x && v[0].y == v[n - 1].y) --n;
+  b = make_double4(INFINITY, INFINITY, -INFINITY, -INFINITY);
+  double s = 0.0, a2 = 0.0, sx = 0.0, sy = 0.0;
+  if (n > 0) {
+    const double2 p0 = v[0];
+    for (int64_t i = 0; i < n; ++i) {
+      const double2 p = v[i];
+      b.x = fmin(b.x, p.x); b.y = fmin(b.y, p.y); b.z = fmax(b.z, p.x); b.w = fmax(b.w, p.y);
+    }
+    if (n >= 3) {
+      for (int64_t i = 1; i < n; ++i) {
+        const double yn = v[i + 1 < n ? i + 1 : 0].y;
+        s = __dadd_rn(s, __dmul_rn(__dsub_rn(v[i].x, p0.x), __dsub_rn(yn, v[i - 1].y)));
+      }
+      for (int64_t i = 1; i + 1 < n; ++i) {
+        const double ax = __dsub_rn(v[i].x, p0.x), ay = __dsub_rn(v[i].y, p0.y);
+        const double bx = __dsub_rn(v[i + 1].x, p0.x), by = __dsub_rn(v[i + 1].y, p0.y);
+        const double cr = __dsub_rn(__dmul_rn(ax, by), __dmul_rn(ay, bx));
+        a2 = __dadd_rn(a2, cr);
+        sx = __dadd_rn(sx, __dmul_rn(cr, __dadd_rn(ax, bx)));
+        sy = __dadd_rn(sy, __dmul_rn(cr, __dadd_rn(ay, by)));
+      }
+    }
+    c = p0;
+    if (a2 != 0.0) {
+      const double den = __dmul_rn(3.0, a2);
+      c = make_double2(__dadd_rn(c.x, __ddiv_rn(sx, den)), __dadd_rn(c.y, __ddiv_rn(sy, den)));
+    }
+  }
+  A = __dmul_rn(s, 0.5);
+  return n;
+}
+
+// One thread per geometry of the polygon layout, rings in layout order (the oracle repeats it in numpy).  Ring r has
+// the area A_r, centroid c_r and box of polygon_props_kernel and the weight w_r = |A_r| for the first ring of a part
+// (its exterior) and -|A_r| for the others (its holes); empty rings are skipped.  With c_f the centroid of the first
+// non-empty ring:
+//   area W = sum w_r (left to right from 0);  centroid = c_f + (sum w_r (c_r - c_f)) / W, or c_f when W == 0;
+//   box = union of the ring boxes;  dist = sqrt(|W| / pi) * ratio.
+// A geometry with one non-empty ring so reproduces polygon_props_kernel bit for bit (|A|, c, box, dist); one with no
+// vertices has area 0, a NaN centroid and the empty box.
+__global__ void polygon_props_multi_kernel(const double2* __restrict__ verts, const int64_t* __restrict__ ring_off,
+                                           const int64_t* __restrict__ part_off, const int64_t* __restrict__ geom_off,
+                                           int64_t n_geom, double ratio, double* __restrict__ area,
+                                           double2* __restrict__ centroid, double4* __restrict__ box, double* __restrict__ dist) {
+  const int64_t gi = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (gi >= n_geom) return;
+  double4 b = make_double4(INFINITY, INFINITY, -INFINITY, -INFINITY);
+  double W = 0.0, nx = 0.0, ny = 0.0;
+  double2 cf = make_double2(NAN, NAN);
+  bool any = false;
+  for (int64_t q = geom_off[gi]; q < geom_off[gi + 1]; ++q) {
+    for (int64_t r = part_off[q]; r < part_off[q + 1]; ++r) {
+      double A;
+      double2 c;
+      double4 rb;
+      if (ring_props(verts + ring_off[r], ring_off[r + 1] - ring_off[r], A, c, rb) == 0) continue;
+      if (!any) { any = true; cf = c; }
+      const double w = r == part_off[q] ? fabs(A) : -fabs(A);
+      b.x = fmin(b.x, rb.x); b.y = fmin(b.y, rb.y); b.z = fmax(b.z, rb.z); b.w = fmax(b.w, rb.w);
+      W = __dadd_rn(W, w);
+      nx = __dadd_rn(nx, __dmul_rn(w, __dsub_rn(c.x, cf.x)));
+      ny = __dadd_rn(ny, __dmul_rn(w, __dsub_rn(c.y, cf.y)));
+    }
+  }
+  if (area) area[gi] = W;
+  if (box) box[gi] = b;
+  if (centroid) centroid[gi] = W != 0.0 ? make_double2(__dadd_rn(cf.x, __ddiv_rn(nx, W)), __dadd_rn(cf.y, __ddiv_rn(ny, W))) : cf;
+  if (dist) dist[gi] = __dmul_rn(__dsqrt_rn(__ddiv_rn(fabs(W), 3.141592653589793)), ratio);
+}
+
 __global__ void pip_emit_kernel(const uint32_t* __restrict__ point, const uint32_t* __restrict__ poly, int64_t E,
                                 int32_t* __restrict__ out, int64_t ld) {
   const int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -290,12 +463,14 @@ namespace sgb {
 namespace {
 
 int pip_count_impl(const char* what, const void* points, int points_f64, int64_t n_points, const double* verts,
-                   const int64_t* ring_off, const double* dist, int64_t n_poly, double xmin, double ymin, double cell, int nx,
-                   int ny, int32_t* total, void* ws, size_t ws_bytes, cudaStream_t stream) {
+                   const int64_t* ring_off, const int64_t* part_off, const int64_t* geom_off, const double* dist, int64_t n_poly,
+                   double xmin, double ymin, double cell, int nx, int ny, int32_t* total, void* ws, size_t ws_bytes,
+                   cudaStream_t stream) {
   SGB_REQUIRE(n_points >= 0 && n_points < (int64_t(1) << 31) && n_poly >= 0 && n_poly < (int64_t(1) << 31), SGB_ERR_RANGE,
               "%s: size out of range", what);
   SGB_REQUIRE(nx >= 1 && ny >= 1 && static_cast<int64_t>(nx) * ny < (int64_t(1) << 28) && cell > 0.0, SGB_ERR_ARG, "%s: bad grid", what);
-  SGB_REQUIRE(total && ws && (n_points == 0 || points) && (n_poly == 0 || (verts && ring_off)), SGB_ERR_ARG, "%s: null tensor", what);
+  SGB_REQUIRE(total && ws && (n_points == 0 || points) && (n_poly == 0 || (verts && ring_off && (!geom_off || part_off))),
+              SGB_ERR_ARG, "%s: null tensor", what);
   SGB_REQUIRE(ws_bytes >= sgb_pip_workspace_bytes(n_points, n_poly, nx, ny), SGB_ERR_WORKSPACE, "%s: workspace too small", what);
   if (n_points == 0 || n_poly == 0) { cudaMemsetAsync(total, 0, sizeof(int32_t), stream); return check_launch(what); }
   const int64_t ncell = static_cast<int64_t>(nx) * ny;
@@ -310,7 +485,15 @@ int pip_count_impl(const char* what, const void* points, int points_f64, int64_t
   if (rc != SGB_OK) return rc;
   if (points_f64) pip_gather_kernel<double><<<nb, 256, 0, stream>>>(static_cast<const double*>(points), w.perm, n_points, w.sorted);
   else pip_gather_kernel<float><<<nb, 256, 0, stream>>>(static_cast<const float*>(points), w.perm, n_points, w.sorted);
-  if (dist)
+  if (geom_off && dist)
+    pip_polygon_kernel<false, true, true><<<static_cast<unsigned>(n_poly), kPipThreads, 0, stream>>>(
+        reinterpret_cast<const double2*>(verts), ring_off, dist, n_poly, w.sorted, w.perm, w.cell_start, g, w.counts, nullptr,
+        nullptr, nullptr, part_off, geom_off);
+  else if (geom_off)
+    pip_polygon_kernel<false, false, true><<<static_cast<unsigned>(n_poly), kPipThreads, 0, stream>>>(
+        reinterpret_cast<const double2*>(verts), ring_off, nullptr, n_poly, w.sorted, w.perm, w.cell_start, g, w.counts, nullptr,
+        nullptr, nullptr, part_off, geom_off);
+  else if (dist)
     pip_polygon_kernel<false, true><<<static_cast<unsigned>(n_poly), kPipThreads, 0, stream>>>(
         reinterpret_cast<const double2*>(verts), ring_off, dist, n_poly, w.sorted, w.perm, w.cell_start, g, w.counts, nullptr,
         nullptr, nullptr);
@@ -324,12 +507,14 @@ int pip_count_impl(const char* what, const void* points, int points_f64, int64_t
   return check_launch(what);
 }
 
-int pip_fill_impl(const char* what, const double* verts, const int64_t* ring_off, const double* dist, int64_t n_points,
-                  int64_t n_poly, double xmin, double ymin, double cell, int nx, int ny, int64_t E, int32_t* edge_index, int64_t ld,
-                  void* ws, size_t ws_bytes, void* scratch, size_t scratch_bytes, cudaStream_t stream) {
+int pip_fill_impl(const char* what, const double* verts, const int64_t* ring_off, const int64_t* part_off, const int64_t* geom_off,
+                  const double* dist, int64_t n_points, int64_t n_poly, double xmin, double ymin, double cell, int nx, int ny,
+                  int64_t E, int32_t* edge_index, int64_t ld, void* ws, size_t ws_bytes, void* scratch, size_t scratch_bytes,
+                  cudaStream_t stream) {
   SGB_REQUIRE(E >= 0 && E < (int64_t(1) << 31), SGB_ERR_RANGE, "%s: E out of range", what);
   if (E == 0) return SGB_OK;
-  SGB_REQUIRE(verts && ring_off && edge_index && ws && scratch && ld >= E, SGB_ERR_ARG, "%s: null tensor", what);
+  SGB_REQUIRE(verts && ring_off && (!geom_off || part_off) && edge_index && ws && scratch && ld >= E, SGB_ERR_ARG,
+              "%s: null tensor", what);
   SGB_REQUIRE(ws_bytes >= sgb_pip_workspace_bytes(n_points, n_poly, nx, ny), SGB_ERR_WORKSPACE, "%s: workspace too small", what);
   SGB_REQUIRE(scratch_bytes >= sgb_pip_fill_scratch_bytes(E), SGB_ERR_WORKSPACE, "%s: scratch too small", what);
   const int64_t ncell = static_cast<int64_t>(nx) * ny;
@@ -341,7 +526,15 @@ int pip_fill_impl(const char* what, const double* verts, const int64_t* ring_off
   uint32_t* pl = reinterpret_cast<uint32_t*>(p); p += eb;
   uint32_t* spt = reinterpret_cast<uint32_t*>(p); p += eb;
   uint32_t* spl = reinterpret_cast<uint32_t*>(p); p += eb;
-  if (dist)
+  if (geom_off && dist)
+    pip_polygon_kernel<true, true, true><<<static_cast<unsigned>(n_poly), kPipThreads, 0, stream>>>(
+        reinterpret_cast<const double2*>(verts), ring_off, dist, n_poly, w.sorted, w.perm, w.cell_start, g, nullptr, w.offsets, pt,
+        pl, part_off, geom_off);
+  else if (geom_off)
+    pip_polygon_kernel<true, false, true><<<static_cast<unsigned>(n_poly), kPipThreads, 0, stream>>>(
+        reinterpret_cast<const double2*>(verts), ring_off, nullptr, n_poly, w.sorted, w.perm, w.cell_start, g, nullptr, w.offsets, pt,
+        pl, part_off, geom_off);
+  else if (dist)
     pip_polygon_kernel<true, true><<<static_cast<unsigned>(n_poly), kPipThreads, 0, stream>>>(
         reinterpret_cast<const double2*>(verts), ring_off, dist, n_poly, w.sorted, w.perm, w.cell_start, g, nullptr, w.offsets, pt, pl);
   else
@@ -364,8 +557,8 @@ int pip_fill_impl(const char* what, const double* verts, const int64_t* ring_off
 extern "C" int sgb_pip_count(const void* points, int points_f64, int64_t n_points, const double* verts, const int64_t* ring_off,
                              int64_t n_poly, double xmin, double ymin, double cell, int nx, int ny, int32_t* total, void* ws,
                              size_t ws_bytes, void* stream) {
-  return pip_count_impl("pip_count", points, points_f64, n_points, verts, ring_off, nullptr, n_poly, xmin, ymin, cell, nx, ny,
-                        total, ws, ws_bytes, static_cast<cudaStream_t>(stream));
+  return pip_count_impl("pip_count", points, points_f64, n_points, verts, ring_off, nullptr, nullptr, nullptr, n_poly, xmin, ymin,
+                        cell, nx, ny, total, ws, ws_bytes, static_cast<cudaStream_t>(stream));
 }
 
 // Pass 2: edge_index [2, E] int32 (row 0 = point index, row 1 = polygon index), point-major, polygon ascending.
@@ -373,8 +566,8 @@ extern "C" int sgb_pip_count(const void* points, int points_f64, int64_t n_point
 extern "C" int sgb_pip_fill(const double* verts, const int64_t* ring_off, int64_t n_points, int64_t n_poly, double xmin, double ymin,
                             double cell, int nx, int ny, int64_t E, int32_t* edge_index, int64_t ld, void* ws, size_t ws_bytes,
                             void* scratch, size_t scratch_bytes, void* stream) {
-  return pip_fill_impl("pip_fill", verts, ring_off, nullptr, n_points, n_poly, xmin, ymin, cell, nx, ny, E, edge_index, ld, ws,
-                       ws_bytes, scratch, scratch_bytes, static_cast<cudaStream_t>(stream));
+  return pip_fill_impl("pip_fill", verts, ring_off, nullptr, nullptr, nullptr, n_points, n_poly, xmin, ymin, cell, nx, ny, E,
+                       edge_index, ld, ws, ws_bytes, scratch, scratch_bytes, static_cast<cudaStream_t>(stream));
 }
 
 // The same two passes against rings grown by dist[poly] (device fp64, one per ring); the grid must cover the union of
@@ -383,8 +576,8 @@ extern "C" int sgb_pip_buffered_count(const void* points, int points_f64, int64_
                                       const int64_t* ring_off, const double* dist, int64_t n_poly, double xmin, double ymin,
                                       double cell, int nx, int ny, int32_t* total, void* ws, size_t ws_bytes, void* stream) {
   SGB_REQUIRE(n_poly <= 0 || dist, SGB_ERR_ARG, "pip_buffered_count: null dist");
-  return pip_count_impl("pip_buffered_count", points, points_f64, n_points, verts, ring_off, dist, n_poly, xmin, ymin, cell, nx,
-                        ny, total, ws, ws_bytes, static_cast<cudaStream_t>(stream));
+  return pip_count_impl("pip_buffered_count", points, points_f64, n_points, verts, ring_off, nullptr, nullptr, dist, n_poly, xmin,
+                        ymin, cell, nx, ny, total, ws, ws_bytes, static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int sgb_pip_buffered_fill(const double* verts, const int64_t* ring_off, const double* dist, int64_t n_points,
@@ -392,8 +585,8 @@ extern "C" int sgb_pip_buffered_fill(const double* verts, const int64_t* ring_of
                                      int32_t* edge_index, int64_t ld, void* ws, size_t ws_bytes, void* scratch,
                                      size_t scratch_bytes, void* stream) {
   SGB_REQUIRE(E == 0 || dist, SGB_ERR_ARG, "pip_buffered_fill: null dist");
-  return pip_fill_impl("pip_buffered_fill", verts, ring_off, dist, n_points, n_poly, xmin, ymin, cell, nx, ny, E, edge_index, ld,
-                       ws, ws_bytes, scratch, scratch_bytes, static_cast<cudaStream_t>(stream));
+  return pip_fill_impl("pip_buffered_fill", verts, ring_off, nullptr, nullptr, dist, n_points, n_poly, xmin, ymin, cell, nx, ny,
+                       E, edge_index, ld, ws, ws_bytes, scratch, scratch_bytes, static_cast<cudaStream_t>(stream));
 }
 
 // Per-ring area / centroid / box and, when `dist` is given, the buffer distance sqrt(|area| / pi) * ratio.
@@ -408,4 +601,44 @@ extern "C" int sgb_polygon_props(const double* verts, const int64_t* ring_off, i
       reinterpret_cast<const double2*>(verts), ring_off, n_poly, ratio, area, reinterpret_cast<double2*>(centroid),
       reinterpret_cast<double4*>(box), dist);
   return check_launch("polygon_props");
+}
+
+// The polygon layout (GeoArrow / cuSpatial): ring_off [R+1] vertices of ring r, part_off [Q+1] rings of part q (its
+// exterior, then its holes), geom_off [n_geom+1] parts of geometry g.  Per geometry: net area (exteriors minus holes),
+// centroid, box (union of the ring boxes) and, when `dist` is given, sqrt(|area| / pi) * ratio.  Outputs as
+// sgb_polygon_props, each may be NULL.
+extern "C" int sgb_polygon_props_multi(const double* verts, const int64_t* ring_off, const int64_t* part_off,
+                                       const int64_t* geom_off, int64_t n_geom, double ratio, double* area, double* centroid,
+                                       double* box, double* dist, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  SGB_REQUIRE(n_geom >= 0 && n_geom < (int64_t(1) << 31), SGB_ERR_RANGE, "polygon_props_multi: size out of range");
+  if (n_geom == 0) return SGB_OK;
+  SGB_REQUIRE(verts && ring_off && part_off && geom_off, SGB_ERR_ARG, "polygon_props_multi: null tensor");
+  polygon_props_multi_kernel<<<static_cast<unsigned>(ceil_div(n_geom, 128)), 128, 0, stream>>>(
+      reinterpret_cast<const double2*>(verts), ring_off, part_off, geom_off, n_geom, ratio, area,
+      reinterpret_cast<double2*>(centroid), reinterpret_cast<double4*>(box), dist);
+  return check_launch("polygon_props_multi");
+}
+
+// The join of sgb_pip_count / _fill (same grid, workspace, scratch and output, with geometries in place of rings)
+// against geometries of the polygon layout: a point is inside geometry g iff the even-odd rule over all rings of g
+// says so.  `dist` [n_geom] (device fp64) or NULL: with it, geometry g is grown by dist[g] as sgb_pip_buffered_count
+// grows one ring, the squared distance taken to the nearest edge of any of its rings; the grid must then cover the
+// geometry boxes grown by |dist| (1 + 2^-20).
+extern "C" int sgb_pip_multi_count(const void* points, int points_f64, int64_t n_points, const double* verts,
+                                   const int64_t* ring_off, const int64_t* part_off, const int64_t* geom_off, const double* dist,
+                                   int64_t n_geom, double xmin, double ymin, double cell, int nx, int ny, int32_t* total,
+                                   void* ws, size_t ws_bytes, void* stream) {
+  SGB_REQUIRE(n_geom <= 0 || (part_off && geom_off), SGB_ERR_ARG, "pip_multi_count: null offsets");
+  return pip_count_impl("pip_multi_count", points, points_f64, n_points, verts, ring_off, part_off, geom_off, dist, n_geom,
+                        xmin, ymin, cell, nx, ny, total, ws, ws_bytes, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int sgb_pip_multi_fill(const double* verts, const int64_t* ring_off, const int64_t* part_off, const int64_t* geom_off,
+                                  const double* dist, int64_t n_points, int64_t n_geom, double xmin, double ymin, double cell,
+                                  int nx, int ny, int64_t E, int32_t* edge_index, int64_t ld, void* ws, size_t ws_bytes,
+                                  void* scratch, size_t scratch_bytes, void* stream) {
+  SGB_REQUIRE(E == 0 || (part_off && geom_off), SGB_ERR_ARG, "pip_multi_fill: null offsets");
+  return pip_fill_impl("pip_multi_fill", verts, ring_off, part_off, geom_off, dist, n_points, n_geom, xmin, ymin, cell, nx, ny,
+                       E, edge_index, ld, ws, ws_bytes, scratch, scratch_bytes, static_cast<cudaStream_t>(stream));
 }

@@ -166,18 +166,19 @@ def setup_prediction_graph(tx, bd, max_k: int, buffer_ratio: float, mode: str = 
     ``mode`` 'cell' / 'nucleus': transcripts strictly inside the outlines of that boundary type, each grown by
     ``sqrt(area / pi) * buffer_ratio`` -- the point-in-polygon join runs on the GPU (``segger_b200.geometry``);
     returns int32 CPU ``[2, E]`` = (transcript row, boundary row) like the reference.  ``bd`` is either a
-    GeoDataFrame (buffered on the host with shapely exactly as the reference does, :229-231), raw outlines as a
-    ``geometry.Outlines`` (rings of the mode's ``boundary_type`` when it is given, renumbered from 0 as the
+    GeoDataFrame (buffered on the host with shapely exactly as the reference does, :229-231; Polygons with holes and
+    MultiPolygons are joined whole, holes and all parts), raw outlines as a ``geometry.Outlines`` (one ring each, or
+    with holes and parts; outlines of the mode's ``boundary_type`` when it is given, renumbered from 0 as the
     reference's ``reset_index(drop=True)`` does, then buffered on the GPU -- no geopandas or shapely needed), or
     outlines that are buffered already: a ``geometry.PackedPolygons`` or a ``(verts, ring_off)`` pair
     (``buffer_ratio`` must then be 0 or None).
     ``mode`` 'uniform': k nearest transcripts of every boundary centroid.  The reference calls
     ``kdtree_neighbors(points, query, max_k)`` without the mandatory ``max_dist`` there and raises TypeError
     (SURVEY Appendix B.4); the evident intent -- no radius cap -- is what this does.  ``bd`` may be the
-    GeoDataFrame, an ``Outlines`` (centroids computed on the GPU) or an [M, 2] centroid array; rows are
+    GeoDataFrame, an ``Outlines`` (centroids computed on the GPU, per geometry) or an [M, 2] centroid array; rows are
     (boundary row, transcript row) as that call returns them.
     """
-    from .geometry import Outlines, PackedPolygons, pack_rings, points_in_polygons
+    from .geometry import Outlines, PackedPolygons, pack_polygons, points_in_polygons
     points = _xy(tx)
     if mode == "uniform":
         if isinstance(bd, Outlines):
@@ -208,7 +209,10 @@ def setup_prediction_graph(tx, bd, max_k: int, buffer_ratio: float, mode: str = 
         polygons = bd[bd["boundary_type"] == boundary_type].geometry
         buffer_dists = np.sqrt(polygons.area / np.pi) * buffer_ratio
         polygons = polygons.buffer(buffer_dists).reset_index(drop=True)
-        polys = PackedPolygons(*pack_rings([np.asarray(g.exterior.coords) for g in polygons]))
+        # every part and hole of the buffered geometries; a frame of one ring per row keeps the one-ring layout
+        verts, ring_off, part_off, geom_off = pack_polygons(polygons)
+        one_ring = np.array_equal(part_off, np.arange(part_off.size)) and np.array_equal(geom_off, np.arange(geom_off.size))
+        polys = PackedPolygons(verts, ring_off) if one_ring else PackedPolygons(verts, ring_off, part_off, geom_off)
         buffer_ratio = 0
     else:
         raise TypeError("setup_prediction_graph: `bd` must be a GeoDataFrame, an Outlines, a PackedPolygons or "
