@@ -1,7 +1,7 @@
 /*
  * libsegger_b200 -- C ABI of the B200-native segger hot path.
  *
- * Every entry point (79) is `extern "C"`, takes plain device pointers and sizes (no torch types),
+ * Every entry point (82) is `extern "C"`, takes plain device pointers and sizes (no torch types),
  * enqueues its work on the `stream` passed in (a cudaStream_t) and returns 0 on success or a
  * negative SGB_ERR_* code; the message is available from sgb_last_error() (thread-local).
  * The library never allocates, frees or retains device memory: outputs and workspaces are
@@ -251,9 +251,23 @@ SGB_API size_t sgb_knn2d_workspace_bytes(const sgb_knn_plan* plan);
 SGB_API int sgb_knn2d(const sgb_knn_plan* plan, const void* points, int is_f64, const void* query /*or NULL*/,
               int64_t* table /*[n_query,k]*/, int32_t* count /*[n_query]*/, void* ws, size_t ws_bytes,
               void* stream);
+/* The same search for any 1 <= k <= 1024 and any max_dist in (0, +inf] (+inf: no radius cap), with the same
+ * outputs, arithmetic and order: KDTree(points).query(q, k, distance_upper_bound) for every k and bound scipy
+ * accepts, and the k nearest transcripts of every boundary centroid of setup_prediction_graph(mode='uniform')
+ * (data/utils/neighbors.py:200-238).  The grid spans the points only and its cell is sized from their density
+ * (no larger than max_dist); a warp per query visits square rings of cells around the query's cell, keeps the
+ * top-k in shared memory and stops once no unscanned point can enter it.  ws64 >= 64 B device; the plan
+ * synchronises the stream once.  k or max_dist out of range -> SGB_ERR_ARG before any CUDA call. */
+SGB_API int sgb_knn2d_ring_plan(const void* points, int is_f64, int64_t n_points, const void* query /*or NULL*/,
+                        int64_t n_query, int k, double max_dist, sgb_knn_plan* plan, void* ws64 /*>=64 B device*/,
+                        void* stream);
+SGB_API size_t sgb_knn2d_ring_workspace_bytes(const sgb_knn_plan* plan);
+SGB_API int sgb_knn2d_ring(const sgb_knn_plan* plan, const void* points, int is_f64, const void* query /*or NULL*/,
+                   int64_t* table /*[n_query,k]*/, int32_t* count /*[n_query]*/, void* ws, size_t ws_bytes,
+                   void* stream);
 /* padded table -> COO (query-major) with offsets = exclusive scan of count: edge_index [2,E] int64
- * contiguous, index_ptr [n_query+1] int64 (knn_to_edge_index, neighbors.py:54-92). total E is
- * returned through *n_edges_host after a stream synchronise when n_edges_host != NULL. */
+ * contiguous, index_ptr [n_query+1] int64 (knn_to_edge_index, neighbors.py:54-92), summed in int64 so it
+ * stays exact past 2^31 edges. total E is returned through *n_edges_host after a stream synchronise when n_edges_host != NULL. */
 SGB_API int sgb_knn_count_valid(const int64_t* table, int64_t n, int k, int64_t pad_value, int32_t* count, void* stream);
 SGB_API size_t sgb_knn_coo_workspace_bytes(int64_t n_query);
 SGB_API int sgb_knn_count_edges(const int32_t* count, int64_t n_query, int64_t* index_ptr, int64_t* n_edges_host,

@@ -101,6 +101,9 @@ _PROTOS = {
     "sgb_knn2d_plan": (c_int, [c_vp, c_int, c_i64, c_vp, c_i64, c_int, C.c_double, C.POINTER(KnnPlan), c_vp, c_vp]),
     "sgb_knn2d_workspace_bytes": (c_sz, [C.POINTER(KnnPlan)]),
     "sgb_knn2d": (c_int, [C.POINTER(KnnPlan), c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
+    "sgb_knn2d_ring_plan": (c_int, [c_vp, c_int, c_i64, c_vp, c_i64, c_int, C.c_double, C.POINTER(KnnPlan), c_vp, c_vp]),
+    "sgb_knn2d_ring_workspace_bytes": (c_sz, [C.POINTER(KnnPlan)]),
+    "sgb_knn2d_ring": (c_int, [C.POINTER(KnnPlan), c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "sgb_knn_count_valid": (c_int, [c_vp, c_i64, c_int, c_i64, c_vp, c_vp]),
     "sgb_knn_coo_workspace_bytes": (c_sz, [c_i64]),
     "sgb_knn_count_edges": (c_int, [c_vp, c_i64, c_vp, C.POINTER(c_i64), c_vp, c_sz, c_vp]),

@@ -12,86 +12,11 @@
 // never push a true neighbour two cells away), sorted by cell with the stable radix sort, and the
 // sorted float64 coordinates are streamed; a query scans 3 rows of 3 adjacent cells, which are 3
 // contiguous ranges of the sorted array.  One thread per query keeps its top-k in registers.
-#include "sgb_api_internal.cuh"
-#include "sgb_sort.cuh"
+// That kernel holds k <= 32 and needs a finite radius; sgb_knn_ring.cu serves every other k <= 1024 and radius.
+#include "sgb_knn.cuh"
 
 namespace sgb {
 namespace {
-
-constexpr int64_t kMaxCells = int64_t(1) << 26;
-
-template <typename T>
-__global__ void __launch_bounds__(256) bbox_kernel(const T* __restrict__ pts, int64_t n, double* __restrict__ box) {
-  // box = [minx, miny, maxx, maxy] pre-initialised; one atomic per CTA via ordered-int trick on doubles
-  __shared__ double sm[4][8];
-  double mnx = INFINITY, mny = INFINITY, mxx = -INFINITY, mxy = -INFINITY;
-  for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < n;
-       i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
-    const double x = static_cast<double>(pts[2 * i]), y = static_cast<double>(pts[2 * i + 1]);
-    mnx = fmin(mnx, x); mny = fmin(mny, y); mxx = fmax(mxx, x); mxy = fmax(mxy, y);
-  }
-#pragma unroll
-  for (int o = 16; o >= 1; o >>= 1) {
-    mnx = fmin(mnx, __shfl_xor_sync(kFull, mnx, o)); mny = fmin(mny, __shfl_xor_sync(kFull, mny, o));
-    mxx = fmax(mxx, __shfl_xor_sync(kFull, mxx, o)); mxy = fmax(mxy, __shfl_xor_sync(kFull, mxy, o));
-  }
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  if (lane == 0) { sm[0][w] = mnx; sm[1][w] = mny; sm[2][w] = mxx; sm[3][w] = mxy; }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    for (int i = 1; i < 8; ++i) {
-      mnx = fmin(mnx, sm[0][i]); mny = fmin(mny, sm[1][i]); mxx = fmax(mxx, sm[2][i]); mxy = fmax(mxy, sm[3][i]);
-    }
-    // order-preserving double <-> signed 64-bit
-    auto enc = [](double d) { long long v = __double_as_longlong(d); return v >= 0 ? v : v ^ 0x7fffffffffffffffLL; };
-    long long* b = reinterpret_cast<long long*>(box);
-    atomicMin(b + 0, enc(mnx)); atomicMin(b + 1, enc(mny)); atomicMax(b + 2, enc(mxx)); atomicMax(b + 3, enc(mxy));
-  }
-}
-__global__ void bbox_init_kernel(double* box) {
-  auto enc = [](double d) { long long v = __double_as_longlong(d); return v >= 0 ? v : v ^ 0x7fffffffffffffffLL; };
-  long long* b = reinterpret_cast<long long*>(box);
-  b[0] = enc(INFINITY); b[1] = enc(INFINITY); b[2] = enc(-INFINITY); b[3] = enc(-INFINITY);
-}
-__global__ void bbox_decode_kernel(double* box) {
-  long long* b = reinterpret_cast<long long*>(box);
-  for (int i = 0; i < 4; ++i) {
-    long long v = b[i];
-    v = v >= 0 ? v : v ^ 0x7fffffffffffffffLL;
-    box[i] = __longlong_as_double(v);
-  }
-}
-
-struct Grid {
-  double xmin, ymin, inv_cell;
-  int nx, ny;
-};
-__device__ __forceinline__ int cell_coord(double v, double lo, double inv, int n) {
-  int c = static_cast<int>(floor((v - lo) * inv));
-  return c < 0 ? 0 : (c >= n ? n - 1 : c);
-}
-
-template <typename T>
-__global__ void cell_key_kernel(const T* __restrict__ pts, int64_t n, Grid g, uint32_t* __restrict__ keys) {
-  const int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const int cx = cell_coord(static_cast<double>(pts[2 * i]), g.xmin, g.inv_cell, g.nx);
-  const int cy = cell_coord(static_cast<double>(pts[2 * i + 1]), g.ymin, g.inv_cell, g.ny);
-  keys[i] = static_cast<uint32_t>(cy) * static_cast<uint32_t>(g.nx) + static_cast<uint32_t>(cx);
-}
-
-template <typename T>
-__global__ void gather_sorted_kernel(const T* __restrict__ pts, const uint32_t* __restrict__ perm, int64_t n,
-                                     double2* __restrict__ sorted) {
-  const int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const int64_t j = perm[i];
-  sorted[i] = make_double2(static_cast<double>(pts[2 * j]), static_cast<double>(pts[2 * j + 1]));
-}
-
-__device__ __forceinline__ bool knn_less(double d1, int i1, double d2, int i2) {
-  return d1 < d2 || (d1 == d2 && i1 < i2);
-}
 
 // K = compile-time capacity of the register top-k (k <= K)
 template <int K, typename T>
@@ -161,10 +86,6 @@ __global__ void count_valid_kernel(const int64_t* __restrict__ table, int64_t n,
   for (int j = 0; j < k; ++j) c += table[r * k + j] != pad ? 1 : 0;
   count[r] = c;
 }
-__global__ void widen_ptr_kernel(const int32_t* __restrict__ in, int64_t n, int64_t* __restrict__ out) {
-  const int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (i < n) out[i] = in[i];
-}
 __global__ void table_to_coo_kernel(const int64_t* __restrict__ table, const int64_t* __restrict__ index_ptr, int64_t n,
                                     int k, int64_t pad, int64_t row_offset, int64_t E, int64_t* __restrict__ ei) {
   const int64_t r = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -180,42 +101,14 @@ __global__ void table_to_coo_kernel(const int64_t* __restrict__ table, const int
   }
 }
 
-struct KnnWs {
-  uint32_t *keys, *skeys, *perm;
-  double2* sorted;
-  int32_t* cell_start;
-  void* sort_ws;
-  size_t sort_bytes, total;
-};
-KnnWs knn_carve(void* ws, int64_t n, int64_t ncells) {
-  KnnWs k{};
-  const size_t nb = align_up(static_cast<size_t>(n > 0 ? n : 1) * 4);
-  char* p = static_cast<char*>(ws);
-  k.keys = reinterpret_cast<uint32_t*>(p); p += nb;
-  k.skeys = reinterpret_cast<uint32_t*>(p); p += nb;
-  k.perm = reinterpret_cast<uint32_t*>(p); p += nb;
-  k.sorted = reinterpret_cast<double2*>(p); p += align_up(static_cast<size_t>(n > 0 ? n : 1) * 16);
-  k.cell_start = reinterpret_cast<int32_t*>(p); p += align_up(static_cast<size_t>(ncells + 1) * 4);
-  k.sort_ws = p;
-  k.sort_bytes = sort_pairs_workspace_bytes(n);
-  k.total = static_cast<size_t>(p - static_cast<char*>(ws)) + k.sort_bytes;
-  return k;
-}
-
 template <typename T>
 int run_knn(const sgb_knn_plan* plan, const T* points, const T* query, int64_t* table, int32_t* count, void* ws,
             cudaStream_t stream) {
   const int64_t n = plan->n_points, nq = plan->n_query;
-  const int64_t ncells = plan->nx * plan->ny;
-  KnnWs w = knn_carve(ws, n, ncells);
+  KnnWs w = knn_carve(ws, n, plan->nx * plan->ny);
   Grid g{plan->xmin, plan->ymin, 1.0 / plan->cell, static_cast<int>(plan->nx), static_cast<int>(plan->ny)};
-  const unsigned nb = static_cast<unsigned>(ceil_div(n, 256));
-  cell_key_kernel<T><<<nb, 256, 0, stream>>>(points, n, g, w.keys);
-  int rc = sort_pairs(w.keys, nullptr, w.skeys, w.perm, n, bits_for(ncells), w.sort_ws, w.sort_bytes, stream);
+  const int rc = bin_points<T>(plan, points, w, g, stream);
   if (rc != SGB_OK) return rc;
-  rc = rowptr_from_sorted(w.skeys, n, w.cell_start, ncells, stream);
-  if (rc != SGB_OK) return rc;
-  gather_sorted_kernel<T><<<nb, 256, 0, stream>>>(points, w.perm, n, w.sorted);
   const unsigned qb = static_cast<unsigned>(ceil_div(nq, 128));
   const double r2 = plan->max_dist * plan->max_dist;
   const int k = plan->k;
@@ -255,22 +148,12 @@ extern "C" int sgb_knn2d_plan(const void* points, int is_f64, int64_t n_points, 
   if (n_points == 0) return SGB_OK;
   SGB_REQUIRE(points && ws64, SGB_ERR_ARG, "knn2d_plan: null tensor");
   double* box = static_cast<double*>(ws64);
-  bbox_init_kernel<<<1, 1, 0, stream>>>(box);
-  const int blocks = sm_count() * 4;
-  if (is_f64) {
-    bbox_kernel<double><<<blocks, 256, 0, stream>>>(static_cast<const double*>(points), n_points, box);
-    if (query && n_query > 0) bbox_kernel<double><<<blocks, 256, 0, stream>>>(static_cast<const double*>(query), n_query, box);
-  } else {
-    bbox_kernel<float><<<blocks, 256, 0, stream>>>(static_cast<const float*>(points), n_points, box);
-    if (query && n_query > 0) bbox_kernel<float><<<blocks, 256, 0, stream>>>(static_cast<const float*>(query), n_query, box);
-  }
-  bbox_decode_kernel<<<1, 1, 0, stream>>>(box);
+  enqueue_bbox(points, n_points, query, n_query, is_f64, box, stream);
   double h[4];
   cudaError_t e = cudaMemcpyAsync(h, box, sizeof(h), cudaMemcpyDeviceToHost, stream);
   if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
   if (e != cudaSuccess) return set_error(SGB_ERR_CUDA, "knn2d_plan: %s", cudaGetErrorString(e));
-  SGB_REQUIRE(h[0] == h[0] && h[2] == h[2] && h[0] > -INFINITY && h[2] < INFINITY && h[1] > -INFINITY && h[3] < INFINITY,
-              SGB_ERR_ARG, "knn2d_plan: non-finite coordinates");
+  SGB_REQUIRE(box_finite(h), SGB_ERR_ARG, "knn2d_plan: non-finite coordinates");
   // enlarge the cell a hair so floor((v - lo) / cell) can never separate true neighbours by 2 cells
   double cell = max_dist * (1.0 + 1e-9);
   const double wx = h[2] - h[0], wy = h[3] - h[1];
@@ -316,25 +199,21 @@ extern "C" int sgb_knn_count_valid(const int64_t* table, int64_t n, int k, int64
   return check_launch("knn_count_valid");
 }
 
-extern "C" size_t sgb_knn_coo_workspace_bytes(int64_t n_query) {
-  return align_up(static_cast<size_t>(n_query + 1) * 4) + scan_workspace_bytes(n_query);
-}
+extern "C" size_t sgb_knn_coo_workspace_bytes(int64_t n_query) { return scan_i64_workspace_bytes(n_query); }
 
 extern "C" int sgb_knn_count_edges(const int32_t* count, int64_t n_query, int64_t* index_ptr, int64_t* n_edges_host,
                                    void* ws, size_t ws_bytes, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   SGB_REQUIRE(n_query >= 0 && index_ptr && ws, SGB_ERR_ARG, "knn_count_edges: bad argument");
   SGB_REQUIRE(ws_bytes >= sgb_knn_coo_workspace_bytes(n_query), SGB_ERR_WORKSPACE, "knn_count_edges: workspace too small");
-  int32_t* p32 = static_cast<int32_t*>(ws);
-  void* scan_ws = static_cast<char*>(ws) + align_up(static_cast<size_t>(n_query + 1) * 4);
   if (n_query == 0) {
-    cudaMemsetAsync(p32, 0, 4, stream);
+    cudaMemsetAsync(index_ptr, 0, sizeof(int64_t), stream);
   } else {
     SGB_REQUIRE(count, SGB_ERR_ARG, "knn_count_edges: null count");
-    int rc = exclusive_scan_i32(count, p32, n_query, scan_ws, scan_workspace_bytes(n_query), stream);
+    // int64 sums: the offsets stay exact when the edge count reaches 2^31 (k = 1024 does at 2.1M queries)
+    int rc = exclusive_scan_i64(count, index_ptr, n_query, ws, ws_bytes, stream);
     if (rc != SGB_OK) return rc;
   }
-  widen_ptr_kernel<<<static_cast<unsigned>(ceil_div(n_query + 1, 256)), 256, 0, stream>>>(p32, n_query + 1, index_ptr);
   if (n_edges_host) {
     cudaError_t e = cudaMemcpyAsync(n_edges_host, index_ptr + n_query, sizeof(int64_t), cudaMemcpyDeviceToHost, stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(stream);

@@ -91,76 +91,81 @@ constexpr int kScanThreads = 256;
 constexpr int kScanItems = 8;
 constexpr int kScanTile = kScanThreads * kScanItems;
 
-__device__ __forceinline__ int block_exclusive_scan(int v, int* total) {
-  __shared__ int wsum[kScanThreads / 32];
-  __shared__ int wtot;
+// A = accumulator / output type: int (the 32-bit scan) or long long (kNN edge offsets that may pass 2^31)
+template <typename A>
+__device__ __forceinline__ A block_exclusive_scan(A v, A* total) {
+  __shared__ A wsum[kScanThreads / 32];
+  __shared__ A wtot;
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  int inc = v;
+  A inc = v;
 #pragma unroll
   for (int o = 1; o < 32; o <<= 1) {
-    const int t = __shfl_up_sync(kFull, inc, o);
+    const A t = __shfl_up_sync(kFull, inc, o);
     if (lane >= o) inc += t;
   }
   if (lane == 31) wsum[w] = inc;
   __syncthreads();
   if (w == 0) {
-    int s = lane < kScanThreads / 32 ? wsum[lane] : 0;
-    int sinc = s;
+    A s = lane < kScanThreads / 32 ? wsum[lane] : 0;
+    A sinc = s;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
-      const int t = __shfl_up_sync(kFull, sinc, o);
+      const A t = __shfl_up_sync(kFull, sinc, o);
       if (lane >= o) sinc += t;
     }
     if (lane < kScanThreads / 32) wsum[lane] = sinc - s;
     if (lane == 31) wtot = sinc;
   }
   __syncthreads();
-  const int res = wsum[w] + inc - v;
+  const A res = wsum[w] + inc - v;
   *total = wtot;
   __syncthreads();
   return res;
 }
 
+template <typename A>
 __global__ void __launch_bounds__(kScanThreads)
-scan_tile_sum_kernel(const int32_t* __restrict__ in, int64_t n, int32_t* __restrict__ bsum) {
+scan_tile_sum_kernel(const int32_t* __restrict__ in, int64_t n, A* __restrict__ bsum) {
   const int64_t base = static_cast<int64_t>(blockIdx.x) * kScanTile + threadIdx.x * kScanItems;
-  int s = 0;
+  A s = 0;
 #pragma unroll
   for (int j = 0; j < kScanItems; ++j)
     if (base + j < n) s += in[base + j];
-  int tot;
-  block_exclusive_scan(s, &tot);
+  A tot;
+  block_exclusive_scan<A>(s, &tot);
   if (threadIdx.x == 0) bsum[blockIdx.x] = tot;
 }
 
 // single CTA: in-place exclusive scan of bsum[0..nb), bsum[nb] = total
+template <typename A>
 __global__ void __launch_bounds__(kScanThreads)
-scan_block_sums_kernel(int32_t* __restrict__ bsum, int64_t nb) {
-  int carry = 0;
+scan_block_sums_kernel(A* __restrict__ bsum, int64_t nb) {
+  A carry = 0;
   for (int64_t base = 0; base < nb; base += kScanThreads) {
     const int64_t i = base + threadIdx.x;
-    const int v = i < nb ? bsum[i] : 0;
-    int tot;
-    const int ex = block_exclusive_scan(v, &tot);
+    const A v = i < nb ? bsum[i] : 0;
+    A tot;
+    const A ex = block_exclusive_scan<A>(v, &tot);
     if (i < nb) bsum[i] = carry + ex;
     carry += tot;
   }
   if (threadIdx.x == 0) bsum[nb] = carry;
 }
 
+template <typename A>
 __global__ void __launch_bounds__(kScanThreads)
-scan_apply_kernel(const int32_t* __restrict__ in, int32_t* __restrict__ out, int64_t n,
-                  const int32_t* __restrict__ bsum, int64_t nb) {
+scan_apply_kernel(const int32_t* __restrict__ in, A* __restrict__ out, int64_t n,
+                  const A* __restrict__ bsum, int64_t nb) {
   const int64_t base = static_cast<int64_t>(blockIdx.x) * kScanTile + threadIdx.x * kScanItems;
   int v[kScanItems];
-  int s = 0;
+  A s = 0;
 #pragma unroll
   for (int j = 0; j < kScanItems; ++j) {
     v[j] = base + j < n ? in[base + j] : 0;
     s += v[j];
   }
-  int tot;
-  int ex = block_exclusive_scan(s, &tot) + bsum[blockIdx.x];
+  A tot;
+  A ex = block_exclusive_scan<A>(s, &tot) + bsum[blockIdx.x];
 #pragma unroll
   for (int j = 0; j < kScanItems; ++j) {
     if (base + j < n) out[base + j] = ex;
@@ -198,27 +203,38 @@ __global__ void presorted_copy_kernel(const uint32_t* __restrict__ keys_in, cons
   }
 }
 
-}  // namespace
-
-size_t scan_workspace_bytes(int64_t n) {
+template <typename A>
+size_t scan_ws_bytes(int64_t n) {
   const int64_t nb = ceil_div(n > 0 ? n : 1, kScanTile);
-  return align_up(static_cast<size_t>(nb + 1) * sizeof(int32_t));
+  return align_up(static_cast<size_t>(nb + 1) * sizeof(A));
 }
 
-int exclusive_scan_i32(const int32_t* in, int32_t* out, int64_t n, void* ws, size_t ws_bytes,
-                       cudaStream_t stream) {
+template <typename A>
+int exclusive_scan(const int32_t* in, A* out, int64_t n, void* ws, size_t ws_bytes, cudaStream_t stream) {
   SGB_REQUIRE(n >= 0 && in && out && ws, SGB_ERR_ARG, "exclusive_scan: null argument");
-  SGB_REQUIRE(ws_bytes >= scan_workspace_bytes(n), SGB_ERR_WORKSPACE, "exclusive_scan: workspace too small");
+  SGB_REQUIRE(ws_bytes >= scan_ws_bytes<A>(n), SGB_ERR_WORKSPACE, "exclusive_scan: workspace too small");
   if (n == 0) {
-    cudaMemsetAsync(out, 0, sizeof(int32_t), stream);
+    cudaMemsetAsync(out, 0, sizeof(A), stream);
     return check_launch("exclusive_scan(memset)");
   }
   const int64_t nb = ceil_div(n, kScanTile);
-  int32_t* bsum = static_cast<int32_t*>(ws);
-  scan_tile_sum_kernel<<<static_cast<unsigned>(nb), kScanThreads, 0, stream>>>(in, n, bsum);
-  scan_block_sums_kernel<<<1, kScanThreads, 0, stream>>>(bsum, nb);
-  scan_apply_kernel<<<static_cast<unsigned>(nb), kScanThreads, 0, stream>>>(in, out, n, bsum, nb);
+  A* bsum = static_cast<A*>(ws);
+  scan_tile_sum_kernel<A><<<static_cast<unsigned>(nb), kScanThreads, 0, stream>>>(in, n, bsum);
+  scan_block_sums_kernel<A><<<1, kScanThreads, 0, stream>>>(bsum, nb);
+  scan_apply_kernel<A><<<static_cast<unsigned>(nb), kScanThreads, 0, stream>>>(in, out, n, bsum, nb);
   return check_launch("exclusive_scan");
+}
+
+}  // namespace
+
+size_t scan_workspace_bytes(int64_t n) { return scan_ws_bytes<int>(n); }
+int exclusive_scan_i32(const int32_t* in, int32_t* out, int64_t n, void* ws, size_t ws_bytes, cudaStream_t stream) {
+  return exclusive_scan<int>(in, out, n, ws, ws_bytes, stream);
+}
+size_t scan_i64_workspace_bytes(int64_t n) { return scan_ws_bytes<long long>(n); }
+int exclusive_scan_i64(const int32_t* in, int64_t* out, int64_t n, void* ws, size_t ws_bytes, cudaStream_t stream) {
+  static_assert(sizeof(long long) == sizeof(int64_t), "int64_t is long long");
+  return exclusive_scan<long long>(in, reinterpret_cast<long long*>(out), n, ws, ws_bytes, stream);
 }
 
 size_t sort_pairs_workspace_bytes(int64_t n) {

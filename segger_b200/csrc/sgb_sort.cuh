@@ -25,6 +25,10 @@ int sort_pairs(const uint32_t* keys_in, const uint32_t* vals_in, uint32_t* keys_
 size_t scan_workspace_bytes(int64_t n);
 int exclusive_scan_i32(const int32_t* in, int32_t* out, int64_t n, void* ws, size_t ws_bytes,
                        cudaStream_t stream);
+// the same scan with int64 sums and output: exact for totals of 2^31 and more
+size_t scan_i64_workspace_bytes(int64_t n);
+int exclusive_scan_i64(const int32_t* in, int64_t* out, int64_t n, void* ws, size_t ws_bytes,
+                       cudaStream_t stream);
 
 // rowptr[r] = lower_bound(sorted_keys, r) for r in [0, n_rows]
 int rowptr_from_sorted(const uint32_t* sorted_keys, int64_t n, int32_t* rowptr, int64_t n_rows,

@@ -3,13 +3,14 @@
 ``knn_to_edge_index`` (:54-92), ``edge_index_to_knn`` is index plumbing and not on the hot path.
 
 Same signatures and return types (CPU ``torch.int64`` edge_index, as scipy + torch produce in the
-reference) -- the search itself runs on the GPU (uniform-grid kNN kernel, float64 distances,
-strict radius, rows ordered by (d^2, index)).  Pass ``device_output=True`` to keep results on the
-device and skip the D2H copy.
+reference) -- the search itself runs on the GPU (uniform-grid kNN kernels, float64 distances,
+strict radius, rows ordered by (d^2, index)) for any k <= 1024 and any radius up to ``inf``.
+Pass ``device_output=True`` to keep results on the device and skip the D2H copy.
 """
 from __future__ import annotations
 
 import ctypes as C
+import math
 from typing import Optional, Tuple
 
 import numpy as np
@@ -37,7 +38,14 @@ def _as_device_points(a, device) -> Tuple[Tensor, bool]:
 
 def knn_table(points, max_k: int, max_dist: float, query=None, device=None) -> Tuple[Tensor, Tensor]:
     """Padded neighbour table [Nq, k] int64 (pad = n_points) and valid counts [Nq] int32, on device.
-    The GPU equivalent of ``KDTree(points, leafsize=100).query(q, k, distance_upper_bound)[1]``."""
+    The GPU equivalent of ``KDTree(points, leafsize=100).query(q, k, distance_upper_bound)[1]`` for
+    1 <= k <= 1024 and 0 < distance_upper_bound <= inf."""
+    # the register kernel holds k <= 32 and needs a finite radius; the ring search takes every other input
+    ring = int(max_k) > 32 or not math.isfinite(max_dist)
+    return _knn_table(points, max_k, max_dist, query, device, ring)
+
+
+def _knn_table(points, max_k: int, max_dist: float, query, device, ring: bool) -> Tuple[Tensor, Tensor]:
     device = torch.device(device if device is not None else "cuda")
     pts, f64 = _as_device_points(points, device)
     qry = None
@@ -46,16 +54,19 @@ def knn_table(points, max_k: int, max_dist: float, query=None, device=None) -> T
         if qf64 != f64:
             pts, qry, f64 = pts.double(), qry.double(), True
     lib = _lib.load()
+    plan_fn, ws_fn, run_fn, name = ((lib.sgb_knn2d_ring_plan, lib.sgb_knn2d_ring_workspace_bytes, lib.sgb_knn2d_ring,
+                                     "knn2d_ring") if ring else
+                                    (lib.sgb_knn2d_plan, lib.sgb_knn2d_workspace_bytes, lib.sgb_knn2d, "knn2d"))
     n, nq = pts.size(0), (qry.size(0) if qry is not None else pts.size(0))
     plan = KnnPlan()
     box = torch.empty(8, dtype=torch.float64, device=device)
-    check(lib.sgb_knn2d_plan(ptr(pts), int(f64), n, ptr(qry), nq, int(max_k), float(max_dist), C.byref(plan),
-                             ptr(box), stream_ptr(device)), "knn2d_plan")
+    check(plan_fn(ptr(pts), int(f64), n, ptr(qry), nq, int(max_k), float(max_dist), C.byref(plan), ptr(box),
+                  stream_ptr(device)), name + "_plan")
     table = torch.empty(nq, max_k, dtype=torch.int64, device=device)
     count = torch.empty(nq, dtype=torch.int32, device=device)
-    ws = torch.empty(max(int(lib.sgb_knn2d_workspace_bytes(C.byref(plan))), 16), dtype=torch.uint8, device=device)
-    check(lib.sgb_knn2d(C.byref(plan), ptr(pts), int(f64), ptr(qry), ptr(table), ptr(count), ptr(ws), ws.numel(),
-                        stream_ptr(device)), "knn2d")
+    ws = torch.empty(max(int(ws_fn(C.byref(plan))), 16), dtype=torch.uint8, device=device)
+    check(run_fn(C.byref(plan), ptr(pts), int(f64), ptr(qry), ptr(table), ptr(count), ptr(ws), ws.numel(),
+                 stream_ptr(device)), name)
     ops._count(14)
     return table, count
 
@@ -101,6 +112,7 @@ def kdtree_neighbors(points: np.ndarray, max_k: int, max_dist: float, chunk_size
                      query: np.ndarray | None = None, device_output: bool = False, device=None):
     """neighbors.py:122-163: kNN (k = max_k, strict radius max_dist) of every query among ``points``
     as a COO edge list, row 0 = query index, row 1 = neighbour index; returns ``(edge_index, None)``.
+    ``max_k`` up to 1024; ``max_dist=np.inf`` means no radius cap, as in scipy.
 
     ``chunk_size`` is accepted for signature compatibility; the whole query set is one launch.
     """
@@ -143,23 +155,6 @@ def setup_transcripts_graph_xy(xy: np.ndarray, max_k: int, max_dist: float) -> T
     return setup_transcripts_graph(xy, max_k, max_dist)
 
 
-def _knn_unbounded(points, query, max_k: int) -> Tensor:
-    """k nearest neighbours without a radius cap on the radius-capped grid kernel: start from the radius that holds
-    ~4k points at the mean density, double it for the queries that found fewer than k until all are full (or the
-    radius covers the whole point set)."""
-    pts = np.asarray(points, dtype=np.float64)
-    n = pts.shape[0]
-    k = min(max_k, n)
-    span = np.maximum(pts.max(0) - pts.min(0), 1e-9)
-    r = float(np.sqrt(4.0 * max(k, 1) * span[0] * span[1] / (np.pi * max(n, 1)))) + 1e-9
-    diag = float(np.hypot(*(np.maximum(pts.max(0), np.asarray(query).max(0)) - np.minimum(pts.min(0), np.asarray(query).min(0))))) + 1.0
-    while True:
-        table, count = knn_table(points, max_k, r, query=query)
-        if r > diag or int((count < k).sum()) == 0:
-            return table
-        r *= 2.0
-
-
 def setup_prediction_graph(tx, bd, max_k: int, buffer_ratio: float, mode: str = "cell", device=None) -> Tensor:
     """neighbors.py:200-238: the tx-neighbors-bd candidate edges.
 
@@ -174,8 +169,8 @@ def setup_prediction_graph(tx, bd, max_k: int, buffer_ratio: float, mode: str = 
     (``buffer_ratio`` must then be 0 or None).
     ``mode`` 'uniform': k nearest transcripts of every boundary centroid.  The reference calls
     ``kdtree_neighbors(points, query, max_k)`` without the mandatory ``max_dist`` there and raises TypeError
-    (SURVEY Appendix B.4); the evident intent -- no radius cap -- is what this does.  ``bd`` may be the
-    GeoDataFrame, an ``Outlines`` (centroids computed on the GPU, per geometry) or an [M, 2] centroid array; rows are
+    (SURVEY Appendix B.4); the evident intent -- no radius cap -- is what this does, in one search on the device.
+    ``bd`` may be the GeoDataFrame, an ``Outlines`` (centroids computed on the GPU, per geometry) or an [M, 2] centroid array; rows are
     (boundary row, transcript row) as that call returns them.
     """
     from .geometry import Outlines, PackedPolygons, pack_polygons, points_in_polygons
@@ -189,10 +184,9 @@ def setup_prediction_graph(tx, bd, max_k: int, buffer_ratio: float, mode: str = 
             query = bd.geometry.centroid.get_coordinates().values
         else:
             query = bd.cpu().numpy() if isinstance(bd, Tensor) else np.asarray(bd)
-        pts = points.cpu().numpy() if isinstance(points, Tensor) else np.asarray(points)
-        table = _knn_unbounded(pts, query, max_k)
         with torch.no_grad():
-            edge_index, _ = _table_to_coo(table, None, int(pts.shape[0]))
+            table, count = knn_table(points, max_k, math.inf, query=query, device=device)
+            edge_index, _ = _table_to_coo(table, count, int(points.shape[0]))
         return edge_index.cpu()
     if mode not in ("cell", "nucleus"):
         raise ValueError(f"setup_prediction_graph: unknown mode '{mode}' (expected 'nucleus', 'cell' or 'uniform')")
